@@ -8,6 +8,11 @@ synthetic conditioning (oracle/inputs.py).  Algorithmic work = 20.28 TFLOP per s
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this framework
   python bench.py --impl reference [--gpus N] ...                # the reference algorithm on the host cores
+  python bench.py ... --dump-outputs DIR                         # also write the last timed step's output as DIR/*.npy
+
+--dump-outputs writes what the timed step returns to its caller, float32, after the timed loop: Stage2Engine.step's
+x_next (rank 0's latent) as x_next.npy, or with --impl reference the network's eps as eps.npy.  The inputs are
+seeded, so two builds run with the same arguments can be compared array for array.
 
 The JSON line's `value` is the BASELINE metric (steps/s, one independent latent per GPU: image sharding, weak
 scaling).  Beside it, in the same line:
@@ -90,11 +95,12 @@ class ClockSampler(threading.Thread):
 # ------------------------------------------------------------------------------------------------
 # reference arm / cpu_baseline: the reference algorithm on the host cores, one FULL step per timing
 # ------------------------------------------------------------------------------------------------
-def cpu_reference(steps: int, warmup: int, sd_cpu=None):
+def cpu_reference(steps: int, warmup: int, sd_cpu=None, dump_dir=None):
     """Times complete stage-2 network steps (control net + UNet, CFG batch 2, 128^2 latent, fp32, every host thread)
-    of the reference algorithm on the CPU: through the reference's own modules imported from /root/reference when
-    that exists (build container; kind "reference"), else through the oracle port of the same functions (GPU box;
-    kind "port").  Shapes are never scaled down; only the repetition count is bounded."""
+    of the reference algorithm on the CPU: through the reference's own modules imported from a reference checkout
+    (oracle/_ref/ or B200SR_REFERENCE_ROOT) when there is one (kind "reference"), else through the oracle port of
+    the same functions (kind "port").  Shapes are never scaled down.  With `dump_dir`, the last timed step's output
+    (the network's eps, 2x4x128x128) is written there as eps.npy."""
     from oracle import configs, inputs, reference_import, sampler as osampler, stage2 as ostage2, weights
 
     torch.set_num_threads(os.cpu_count() or 1)
@@ -127,8 +133,10 @@ def cpu_reference(steps: int, warmup: int, sd_cpu=None):
         step()
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
+        out = step()
     dt = (time.perf_counter() - t0) / steps
+    if dump_dir:
+        dump_outputs(dump_dir, {"eps": out})
     return {"value": 1.0 / dt, "unit": UNIT, "cores": torch.get_num_threads(), "kind": kind,
             "sample": f"{steps} full step(s) of the workload (20.28 TFLOP each, fp32) after {warmup} warm-up step(s); "
                       f"{dt:.2f} s per step; no extrapolation",
@@ -138,9 +146,8 @@ def cpu_reference(steps: int, warmup: int, sd_cpu=None):
 def run_reference(args, rank: int):
     if rank != 0:
         return
-    k = max(1, min(args.steps, 2))
-    w = 1 if args.warmup > 0 else 0
-    base = cpu_reference(k, w)
+    k, w = args.steps, args.warmup
+    base = cpu_reference(k, w, dump_dir=args.dump_outputs)
     line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": k, "warmup": w, "ms_per_step": 1000.0 / base["value"], "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -335,6 +342,15 @@ def images_block(wrapper, dev, rank: int, world: int, per_rank: int, upscale: in
             "rank0_cache_misses_per_image": r["misses"]}
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each tensor whole as out_dir/<name>.npy in float32 (the step's latent is 1x4x128x128: 256 KB)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().to("cpu", torch.float32).numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 # this framework
 # ------------------------------------------------------------------------------------------------
@@ -380,10 +396,13 @@ def run_b200(args, rank: int, world: int, local_rank: int):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        eng.step(x, step_i, noise, 0.0, copy_out=False)
+        out, _ = eng.step(x, step_i, noise, 0.0, copy_out=False)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs and rank == 0:
+        # `out` is the engine's output buffer, which the next step overwrites: copy it out now
+        dump_outputs(args.dump_outputs, {"x_next": out})
     # ---- end-to-end timing: host buffers, H2D + D2H inside the timed region ----------------------
     barrier()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -557,7 +576,11 @@ def main():
     ap.add_argument("--tiled-steps", type=int, default=2, help="timed tiled sampler steps")
     ap.add_argument("--tile-batch", type=int, default=1, help="windows per network call")
     ap.add_argument("--images-per-rank", type=int, default=2, help="config-5 sample: images per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's output (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,4 +1,4 @@
-"""ORACLE tooling — run in the BUILD container (needs /root/reference):
+"""ORACLE tooling — needs a checkout of the reference project at oracle/_ref/ (or B200SR_REFERENCE_ROOT):
 
     python -m oracle.make_golden
 
@@ -318,7 +318,7 @@ def keys():
 
 
 if __name__ == "__main__":
-    assert reference_import.available(), "needs /root/reference"
+    assert reference_import.available(), "needs a reference checkout at oracle/_ref/ or B200SR_REFERENCE_ROOT"
     os.makedirs(GOLDEN, exist_ok=True)
     torch.set_grad_enabled(False)
     keys()

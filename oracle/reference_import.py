@@ -1,5 +1,6 @@
-"""ORACLE tooling — import the *real* reference modules from /root/reference (build container
-only; the GPU box has no /root/reference) to pin the restatement and to generate tests/golden/.
+"""ORACLE tooling — import the *real* reference modules from a checkout of the reference project
+(B200SR_REFERENCE_ROOT, default oracle/_ref/, which git ignores) to pin the restatement and to generate
+tests/golden/.  Without such a checkout, available() is False and the tests that need it skip.
 
 Three third-party packages the reference imports at module scope are absent from this image and
 are not executed on the denoiser path; they are replaced by empty stubs (SURVEY.md Appendix B):
@@ -12,7 +13,7 @@ import types
 
 import torch
 
-REFERENCE_ROOT = os.environ.get("B200SR_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("B200SR_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 def available() -> bool:
