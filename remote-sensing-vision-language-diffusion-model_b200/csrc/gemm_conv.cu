@@ -115,7 +115,8 @@ struct GemmParams {
   // mode 0, LayerNorm folded around the GEMM (see b200sr_epilogue in include/b200sr.h):
   //   consumer  v = rstd[m] * (acc[m, n] - mean[m] * colsum[g, n]) + shift[g, n]   with (mean, rstd) folded from ln_parts
   //             per-row partial (sum, sum of squares) written by the GEMM that produced A
-  //   producer  ln_stats_out[n_blk][m] = (sum, sum of squares) of the bf16 values this tile stores in row m
+  //   producer  ln_stats_out[n_blk][m] = (sum, sum of squares) of row m's fp32 values in this tile, before their rounding
+  //             to the bf16 values it stores
   const float2* ln_stats;   // [ln_parts][M], nullptr = off
   int ln_parts;
   const float* ln_colsum;   // [weight groups][N]

@@ -16,8 +16,10 @@ namespace b200sr {
 
 static constexpr int GN_WS_COUNTER_FLOATS = 256;
 
-// sums in fp64 -> (mean, 1/sqrt(var + eps)); the variance is formed in fp64 (no cancellation), only the
-// final reciprocal square root is fp32 (correctly rounded sqrt and divide).
+// (sum, sum of squares) of a group -> (mean, 1/sqrt(var + eps)).  The sums arrive as fp64 folds of fp32 partials: each
+// thread sums its pixels in fp32 and each CTA its threads' sums in fp32, so those partials carry fp32 rounding error;
+// only the fold across chunks and E[x^2] - mean^2 are fp64 (rounding negligible next to the partials'), and the final reciprocal square
+// root is fp32 (correctly rounded sqrt and divide).
 __device__ __forceinline__ float2 gn_mean_rstd(double sum, double sumsq, double inv_cnt, float eps) {
   const double mean = sum * inv_cnt;
   double var = sumsq * inv_cnt - mean * mean;
