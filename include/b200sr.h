@@ -270,6 +270,21 @@ int b200sr_wavelet_level(const float* img, float* low, float* high, int32_t firs
 int b200sr_add_f32(const float* a, const float* b, float* out, int64_t n, void* stream);
 int b200sr_image_to_u8(const float* x, void* out, int32_t C, int32_t H, int32_t W, int32_t OH, int32_t OW, void* stream);
 
+/* Stage-1 -> stage-2 hand-off (infer.py:133-138 tensor2img; models/util.py:132-156 PIL2Tensor), uint8 images HWC:
+ *   tensor2img_u8:    fp32 [C, H, W] -> uint8 [H, W, C]: t = (clamp(x, -1, 1) + 1) / 2 in fp32, rint(t * 255) in fp32
+ *                     (round half to even, as numpy .round()); SR3's tensor2img, utils/tensor2img.py:4-21
+ *   resample_u8:      one axis of PIL.Image.resize(..., Image.BICUBIC) (libImaging/Resample.c, 8 bits per channel):
+ *                     src viewed as [outer, in_len, inner] bytes -> dst [outer, out_len, inner]; the horizontal pass
+ *                     of an [H, W, C] image is (outer, inner) = (H, C), the vertical pass (1, W * C).  bounds int32
+ *                     [out_len, 2] = (first tap, tap count), coeffs int32 [out_len, ksize] in 22-bit fixed point,
+ *                     both built on the host (b200sr.ops.pillow_bicubic_tables); dst[o] = clamp((2^21 + sum of
+ *                     src * coeff) >> 22, 0, 255).  src and dst must not overlap.
+ *   img_u8_to_tensor: uint8 [H, W, C] -> fp32 [C, H, W]: (float)(x / 255.0 * 2.0 - 1.0) evaluated in double */
+int b200sr_tensor2img_u8(const float* x, void* out, int32_t C, int32_t H, int32_t W, void* stream);
+int b200sr_resample_u8(const void* src, void* dst, int32_t outer, int32_t in_len, int32_t out_len, int32_t inner,
+                       const int32_t* bounds, const int32_t* coeffs, int32_t ksize, void* stream);
+int b200sr_img_u8_to_tensor(const void* in, float* out, int32_t C, int32_t H, int32_t W, void* stream);
+
 /* Up to 8 small device-to-device copies in one launch (bytes % 4 == 0, 4-byte aligned): the per-step loader of
  * the sampler engine (latent, noise, this step's row of the scalar table sampling.py:598-606 and of the
  * precomputed timestep-embedding projections openaimodel.py:281-287) into the buffers a CUDA graph reads. */

@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # B200SR_LIB selects another in-tree build of the same ABI (A/B kernel experiments); default = the product library
 LIB_PATH = os.path.join(_HERE, os.environ.get("B200SR_LIB", "libb200sr.so"))
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 c_void_p, c_int, c_i64, c_float, c_size_t = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
 
@@ -121,6 +121,9 @@ SIGNATURES = {
     "b200sr_wavelet_level": (c_int, [P, P, P, c_int, c_int, c_int, c_int, c_int, P]),
     "b200sr_add_f32": (c_int, [P, P, P, c_i64, P]),
     "b200sr_image_to_u8": (c_int, [P, P, c_int, c_int, c_int, c_int, c_int, P]),
+    "b200sr_tensor2img_u8": (c_int, [P, P, c_int, c_int, c_int, P]),
+    "b200sr_resample_u8": (c_int, [P, P, c_int, c_int, c_int, c_int, P, P, c_int, P]),
+    "b200sr_img_u8_to_tensor": (c_int, [P, P, c_int, c_int, c_int, P]),
     "b200sr_copy_batch": (c_int, [C.POINTER(Copy), c_int, P]),
     "b200sr_tile_weighted_strip": (c_int, [P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]),
     "b200sr_strip_add": (c_int, [P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]),

@@ -13,8 +13,10 @@ There is no CPU path and no torch fallback here: tensors that are not CUDA tenso
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Optional
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -837,4 +839,118 @@ def image_to_u8(x: torch.Tensor, oh: int, ow: int) -> torch.Tensor:
     c, h, w = x.shape
     out = torch.empty(oh, ow, c, dtype=torch.uint8, device=x.device)
     check(_lib.load().b200sr_image_to_u8(x.data_ptr(), out.data_ptr(), c, h, w, oh, ow, _stream()), "image_to_u8")
+    return out
+
+
+# ------------------------------------------------------------------------------------------------
+# stage-1 -> stage-2 hand-off: tensor2img, PIL2Tensor's Image.resize(BICUBIC) and uint8 -> [-1, 1]
+# ------------------------------------------------------------------------------------------------
+PILLOW_PRECISION_BITS = 22
+
+
+def _pillow_bicubic(x):
+    """libImaging/Resample.c bicubic_filter (a = -0.5, support 2), float64, same operation order."""
+    a = -0.5
+    x = np.abs(x)
+    near = ((a + 2.0) * x - (a + 3.0)) * x * x + 1
+    far = (((x - 5) * x + 8) * x - 4) * a
+    return np.where(x < 1.0, near, np.where(x < 2.0, far, 0.0))
+
+
+def pillow_bicubic_tables(in_len: int, out_len: int):
+    """Pillow's precompute_coeffs + normalize_coeffs_8bpc (libImaging/Resample.c) for one axis of
+    ``Image.resize(..., Image.BICUBIC)`` over the whole image (box = (0, in_len)), as numpy arrays:
+    (bounds int32 [out_len, 2] = (first tap, tap count), coeffs int32 [out_len, ksize], ksize).
+
+    Per output index o: center = (o + 0.5) * scale with scale = in / out; the filter is stretched by
+    fs = max(scale, 1) (antialiasing when reducing); taps xmin .. xmin + n - 1 with xmin = int(center - support + 0.5)
+    and support = 2 * fs; w_k = filter((k + xmin - center + 0.5) * (1 / fs)), divided by their sequential double sum
+    (unless it is 0); the fixed-point coefficient is w * 2^22 rounded half away from zero."""
+    if in_len <= 0 or out_len <= 0:
+        raise ValueError(f"resample lengths must be positive, got {in_len} -> {out_len}")
+    scale = float(in_len) / out_len
+    fs = max(scale, 1.0)
+    support = 2.0 * fs
+    ksize = int(math.ceil(support)) * 2 + 1
+    center = (np.arange(out_len, dtype=np.float64) + 0.5) * scale
+    xmin = np.maximum((center - support + 0.5).astype(np.int64), 0)           # C (int) cast: toward zero
+    xmax = np.minimum((center + support + 0.5).astype(np.int64), in_len)
+    n = xmax - xmin
+    k = np.arange(ksize, dtype=np.int64)
+    pos = (k[None, :] + xmin[:, None]).astype(np.float64)
+    w = _pillow_bicubic((pos - center[:, None] + 0.5) * (1.0 / fs))
+    w = np.where(k[None, :] < n[:, None], w, 0.0)
+    ww = np.zeros(out_len, dtype=np.float64)
+    for j in range(ksize):                                                      # sequential sum, as the C loop
+        ww = ww + w[:, j]
+    w = np.where(ww[:, None] != 0.0, w / np.where(ww == 0.0, 1.0, ww)[:, None], w)
+    one = float(1 << PILLOW_PRECISION_BITS)
+    fixed = np.where(w < 0, (-0.5 + w * one).astype(np.int64), (0.5 + w * one).astype(np.int64))
+    bounds = np.stack((xmin, n), 1).astype(np.int32)
+    return bounds, fixed.astype(np.int32), ksize
+
+
+_resample_tables: dict = {}
+
+
+def _device_tables(in_len: int, out_len: int, device: torch.device):
+    key = (in_len, out_len, device.type, device.index)
+    t = _resample_tables.get(key)
+    if t is None:
+        bounds, coeffs, ksize = pillow_bicubic_tables(in_len, out_len)
+        t = (torch.from_numpy(bounds).to(device), torch.from_numpy(coeffs).to(device), ksize)
+        _resample_tables[key] = t
+    return t
+
+
+def tensor2img_u8(x: torch.Tensor) -> torch.Tensor:
+    """fp32 [C, H, W] in [-1, 1] -> uint8 [H, W, C]: rint((clamp(x, -1, 1) + 1) / 2 * 255) in fp32."""
+    _req(x, torch.float32, "tensor2img_u8.x")
+    c, h, w = x.shape
+    out = torch.empty(h, w, c, dtype=torch.uint8, device=x.device)
+    check(_lib.load().b200sr_tensor2img_u8(x.data_ptr(), out.data_ptr(), c, h, w, _stream()), "tensor2img_u8")
+    return out
+
+
+def resample_u8_axis(src: torch.Tensor, out_len: int, axis: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """One Pillow bicubic pass of a uint8 [H, W, C] image along axis 1 (width) or 0 (height).  `out` (optional) is
+    the destination; its shape must be the result's."""
+    _req(src, torch.uint8, "resample_u8.src")
+    h, w, c = src.shape
+    if axis == 1:
+        outer, in_len, inner, shape = h, w, c, (h, out_len, c)
+    elif axis == 0:
+        outer, in_len, inner, shape = 1, h, w * c, (out_len, w, c)
+    else:
+        raise ValueError("axis must be 0 (height) or 1 (width)")
+    if out is None:
+        out = torch.empty(shape, dtype=torch.uint8, device=src.device)
+    elif tuple(out.shape) != shape:
+        raise ValueError(f"resample_u8: out has shape {tuple(out.shape)}, expected {shape}")
+    _req(out, torch.uint8, "resample_u8.out")
+    bounds, coeffs, ksize = _device_tables(in_len, out_len, src.device)
+    check(_lib.load().b200sr_resample_u8(src.data_ptr(), out.data_ptr(), outer, in_len, out_len, inner,
+                                         bounds.data_ptr(), coeffs.data_ptr(), ksize, _stream()), "resample_u8")
+    return out
+
+
+def resize_bicubic_u8(img: torch.Tensor, oh: int, ow: int) -> torch.Tensor:
+    """``PIL.Image.fromarray(img).resize((ow, oh), Image.BICUBIC)`` of a uint8 [H, W, C] image, byte for byte: the
+    horizontal pass first (when the width changes), then the vertical pass (when the height changes); an unchanged
+    size is a copy."""
+    _req(img, torch.uint8, "resize_bicubic_u8.img")
+    h, w, _ = img.shape
+    if ow != w:
+        img = resample_u8_axis(img, ow, 1)
+    if oh != h:
+        img = resample_u8_axis(img, oh, 0)
+    return img.clone() if (oh, ow) == (h, w) else img
+
+
+def img_u8_to_tensor(img: torch.Tensor) -> torch.Tensor:
+    """uint8 [H, W, C] -> fp32 [C, H, W]: (float)(x / 255 * 2 - 1) computed in double."""
+    _req(img, torch.uint8, "img_u8_to_tensor.img")
+    h, w, c = img.shape
+    out = torch.empty(c, h, w, dtype=torch.float32, device=img.device)
+    check(_lib.load().b200sr_img_u8_to_tensor(img.data_ptr(), out.data_ptr(), c, h, w, _stream()), "img_u8_to_tensor")
     return out

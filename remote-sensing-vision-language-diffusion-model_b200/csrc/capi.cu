@@ -145,6 +145,10 @@ int wavelet_level(const float* img, float* low, float* high, int first, int BC, 
                   cudaStream_t stream);
 int add_f32(const float* a, const float* b, float* out, long long n, cudaStream_t stream);
 int image_to_u8(const float* x, void* out, int C, int H, int W, int OH, int OW, cudaStream_t stream);
+int tensor2img_u8(const float* x, void* out, int C, int H, int W, cudaStream_t stream);
+int resample_u8(const void* src, void* dst, int outer, int in_len, int out_len, int inner, const int* bounds,
+                const int* coeffs, int ksize, cudaStream_t stream);
+int img_u8_to_tensor(const void* in, float* out, int C, int H, int W, cudaStream_t stream);
 int copy_batch(const void* const* src, void* const* dst, const long long* bytes, int n, cudaStream_t stream);
 int tile_weighted_strip(const float* tile, const float* weight, float* strip, int BC, int th, int tw, int y0, int x0,
                         int sh, int sw, cudaStream_t stream);
@@ -191,7 +195,7 @@ using namespace b200sr;
 
 extern "C" {
 
-int b200sr_abi_version(void) { return 5; }
+int b200sr_abi_version(void) { return 6; }
 int b200sr_num_sms(void) {
   int dev = 0, n = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return B200SR_ENODEV;
@@ -381,6 +385,19 @@ int b200sr_add_f32(const float* a, const float* b, float* out, int64_t n, void* 
 int b200sr_image_to_u8(const float* x, void* out, int32_t C, int32_t H, int32_t W, int32_t OH, int32_t OW, void* stream) {
   if (x == nullptr || out == nullptr) return B200SR_EINVAL;
   return image_to_u8(x, out, C, H, W, OH, OW, S(stream));
+}
+int b200sr_tensor2img_u8(const float* x, void* out, int32_t C, int32_t H, int32_t W, void* stream) {
+  if (x == nullptr || out == nullptr) return B200SR_EINVAL;
+  return tensor2img_u8(x, out, C, H, W, S(stream));
+}
+int b200sr_resample_u8(const void* src, void* dst, int32_t outer, int32_t in_len, int32_t out_len, int32_t inner,
+                       const int32_t* bounds, const int32_t* coeffs, int32_t ksize, void* stream) {
+  if (src == nullptr || dst == nullptr || bounds == nullptr || coeffs == nullptr) return B200SR_EINVAL;
+  return resample_u8(src, dst, outer, in_len, out_len, inner, bounds, coeffs, ksize, S(stream));
+}
+int b200sr_img_u8_to_tensor(const void* in, float* out, int32_t C, int32_t H, int32_t W, void* stream) {
+  if (in == nullptr || out == nullptr) return B200SR_EINVAL;
+  return img_u8_to_tensor(in, out, C, H, W, S(stream));
 }
 
 }  // extern "C"
