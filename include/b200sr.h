@@ -27,6 +27,7 @@ extern "C" {
 #endif
 
 /* Library / device introspection. */
+#define B200SR_ABI_VERSION 6  /* what b200sr_abi_version() returns */
 int b200sr_abi_version(void);         /* bumps on any signature change */
 int b200sr_num_sms(void);             /* SM count of the current device, <0 on error */
 

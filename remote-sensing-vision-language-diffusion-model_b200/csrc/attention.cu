@@ -439,17 +439,24 @@ static AttnPlan attention_plan(int B, int H, int Nq, int Nk) {
   return a;
 }
 
-size_t attention_d64_workspace_bytes(int B, int H, int Nq, int Nk) {
+}  // namespace b200sr
+
+using namespace b200sr;
+
+extern "C" size_t b200sr_attention_d64_workspace_bytes(int32_t B, int32_t H, int32_t Nq, int32_t Nk) {
   if (B <= 0 || H <= 0 || Nq <= 0 || Nk <= 0) return 0;
   return attention_plan(B, H, Nq, Nk).workspace_bytes;
 }
 
 // q: [B, Nq, ldq] window at q_col; k, v: [B, Nk, ldk / ldv] windows; out: [B, Nq, ldo], head h at h*64.
-// workspace: attention_d64_workspace_bytes() bytes (may be null when that is 0); its first 2 KiB are
+// workspace: b200sr_attention_d64_workspace_bytes() bytes (may be null when that is 0); its first 2 KiB are
 // arrival counters that must be zero before the first call and are left zero by every call.
-int attention_d64(const void* q, long long ldq, int q_col, const void* k, long long ldk, int k_col, const void* v,
-                  long long ldv, int v_col, void* out, long long ldo, int B, int H, int Nq, int Nk, float scale,
-                  int causal, void* workspace, cudaStream_t stream) {
+extern "C" int b200sr_attention_d64(const void* q, int64_t ldq, int32_t q_col, const void* k, int64_t ldk, int32_t k_col,
+                                    const void* v, int64_t ldv, int32_t v_col, void* out, int64_t ldo, int32_t B, int32_t H,
+                                    int32_t Nq, int32_t Nk, float scale, int32_t causal, void* workspace,
+                                    void* stream_ptr) {
+  if (q == nullptr || k == nullptr || v == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (B <= 0 || H <= 0 || Nq <= 0 || Nk <= 0) return B200SR_EINVAL;
   if (causal && (Nq != Nk || Nk > ATT_BN)) return B200SR_EINVAL;   // causal: self-attention within one key block (77 tokens)
   if ((ldq % 8) || (ldk % 8) || (ldv % 8) || (ldo % 8) || (q_col % 8) || (k_col % 8) || (v_col % 8))
@@ -498,8 +505,6 @@ int attention_d64(const void* q, long long ldq, int q_col, const void* k, long l
              ? B200SR_OK
              : B200SR_ELAUNCH;
 }
-
-}  // namespace b200sr
 
 #ifdef B200SR_ATT_TRACE
 extern "C" void b200sr_debug_set_attn_trace(void* p) { b200sr::g_att_trace = reinterpret_cast<long long*>(p); }

@@ -2,6 +2,8 @@
 // tcgen05/TMEM, UMMA descriptors) and small host utilities.  Everything here is written
 // for Blackwell only; there is no fallback path.
 #pragma once
+// The C ABI: every .cu file defines its extern "C" entry points against these prototypes.
+#include "../../include/b200sr.h"
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -383,37 +385,5 @@ int make_tmap_f32(CUtensorMap* out, const void* base, int rank, const uint64_t* 
                   const uint32_t* box);   // fp32 elements, 128B swizzle (box row = 32 floats)
 int make_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                    const uint32_t* box, int swizzle_bytes = 128);
-
-// Fused GEMM / convolution epilogue (mirror of b200sr_epilogue in include/b200sr.h).
-struct EpilogueArgs {
-  const float* bias;
-  const float* rowvec;
-  int rows_per_group;
-  long long ld_rowvec;  // 0 = N
-  const void* residual;
-  long long ldr;
-  void* out;
-  long long ldc;
-  int out_fp32;
-  int geglu;
-  float alpha;
-  int act;  // 0 = none, 1 = SiLU, 2 = GELU (erf), 3 = quick GELU (applied last)
-  int softmax_valid;        // > 0: epilogue = row softmax over each 80-column segment (first softmax_valid columns)
-  int w_dynamic;            // != 0: the W operand is produced by an earlier kernel (no prefetch ahead of griddepcontrol.wait)
-  int w_rows_per_group;     // > 0: rows [g * w_rows_per_group, ...) of A use weight rows offset by g * w_group_stride
-  long long w_group_stride;
-  const float* a_gn_stats;  // conv3x3 (halo path) only: GroupNorm(+SiLU) of the input fused into the A tile
-  const float* a_gn_weight;
-  const float* a_gn_bias;
-  int a_gn_groups, a_gn_silu;
-  const float* ln_stats;    // GEMM only: LayerNorm of the A rows folded into the epilogue (see include/b200sr.h)
-  int ln_parts;
-  const float* ln_colsum;
-  const float* ln_shift;
-  float ln_eps;
-  float* ln_stats_out;      // GEMM only: per-row partial (sum, sum of squares) of the stored bf16 output, [n tiles][M][2]
-  int row_softmax;          // GEMM only: two-pass softmax over whole rows (1 = statistics pass, 2 = apply pass)
-  int row_softmax_valid;
-};
 
 }  // namespace b200sr

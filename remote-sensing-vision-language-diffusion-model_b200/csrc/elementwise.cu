@@ -63,18 +63,33 @@ __global__ void nhwc_bf16_to_nchw_f32_kernel(const __nv_bfloat16* __restrict__ x
   }
 }
 
-int nchw_f32_to_nhwc_bf16(const float* x, void* y, int N, int C, int HW, float scale, cudaStream_t stream) {
+}  // namespace b200sr
+
+using namespace b200sr;
+
+extern "C" int b200sr_nchw_f32_to_nhwc_bf16(const float* x, void* y, int32_t N, int32_t C, int32_t HW, float scale,
+                                            void* stream_ptr) {
+  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (N <= 0 || C <= 0 || HW <= 0) return B200SR_EINVAL;
   dim3 grid((HW + 31) / 32, (C + 31) / 32, N), block(32, 8);
   launch_k(nchw_f32_to_nhwc_bf16_kernel, dim3(grid), dim3(block), 0, stream, 1, x, reinterpret_cast<__nv_bfloat16*>(y), C, HW, scale);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
-int nhwc_bf16_to_nchw_f32(const void* x, float* y, int N, int C, int Cs, int HW, cudaStream_t stream) {
+extern "C" int b200sr_nhwc_bf16_to_nchw_f32_strided(const void* x, float* y, int32_t N, int32_t C, int32_t Cs,
+                                                    int32_t HW, void* stream_ptr) {
+  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (N <= 0 || C <= 0 || HW <= 0 || Cs < C) return B200SR_EINVAL;
   dim3 grid((HW + 31) / 32, (C + 31) / 32, N), block(32, 8);
   launch_k(nhwc_bf16_to_nchw_f32_kernel, dim3(grid), dim3(block), 0, stream, 1, reinterpret_cast<const __nv_bfloat16*>(x), y, C, Cs, HW);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+extern "C" int b200sr_nhwc_bf16_to_nchw_f32(const void* x, float* y, int32_t N, int32_t C, int32_t HW, void* stream) {
+  return b200sr_nhwc_bf16_to_nchw_f32_strided(x, y, N, C, C, HW, stream);
+}
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // nearest 2x upsample, NHWC bf16, 16-byte vectors
@@ -94,7 +109,13 @@ __global__ void upsample2x_kernel(const uint4* __restrict__ x, uint4* __restrict
     y[i] = __ldg(x + ((n * H + (oh >> 1)) * W + (ow >> 1)) * C8 + cv);
   }
 }
-int upsample2x_nhwc(const void* x, void* y, int N, int H, int W, int C, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_upsample2x_nhwc(const void* x, void* y, int32_t N, int32_t H, int32_t W, int32_t C,
+                                      void* stream_ptr) {
+  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (N <= 0 || H <= 0 || W <= 0 || C <= 0 || (C % 8)) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(N) * 4 * H * W * (C / 8);
   int grid = static_cast<int>((total + 255) / 256);
@@ -103,6 +124,8 @@ int upsample2x_nhwc(const void* x, void* y, int N, int H, int W, int C, cudaStre
                                               C / 8, total);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // out[:, :Ca] = a ; out[:, Ca:] = b (+ c)       rows of Ca / Cb channels, bf16, 16-byte vectors
@@ -137,8 +160,13 @@ __global__ void concat_add_kernel(const uint4* __restrict__ a, const uint4* __re
     out[i] = v;
   }
 }
-int concat_add(const void* a, int Ca, const void* b, int Cb, const void* c, void* out, long long rows,
-               cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_concat_add(const void* a, int32_t Ca, const void* b, int32_t Cb, const void* c, void* out,
+                                 int64_t rows, void* stream_ptr) {
+  if ((a == nullptr && Ca > 0) || b == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (rows <= 0 || Ca < 0 || Cb <= 0 || (Ca % 8) || (Cb % 8)) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(rows) * ((Ca + Cb) / 8);
   int grid = static_cast<int>((total + 255) / 256);
@@ -148,6 +176,8 @@ int concat_add(const void* a, int Ca, const void* b, int Cb, const void* c, void
                                               Cb / 8, static_cast<size_t>(rows));
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // y = a + alpha * b (bf16), used for residual adds that could not be fused
@@ -162,7 +192,12 @@ __global__ void axpy_bf16_kernel(const __nv_bfloat162* __restrict__ a, const __n
     y[i] = __floats2bfloat162_rn(f.x + alpha * g.x, f.y + alpha * g.y);
   }
 }
-int axpy_bf16(const void* a, const void* b, void* y, float alpha, long long n, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_axpy_bf16(const void* a, const void* b, void* y, float alpha, int64_t n, void* stream_ptr) {
+  if (a == nullptr || b == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (n <= 0 || (n & 1)) return B200SR_EINVAL;
   const size_t n2 = static_cast<size_t>(n) / 2;
   int grid = static_cast<int>((n2 + 255) / 256);
@@ -172,6 +207,8 @@ int axpy_bf16(const void* a, const void* b, void* y, float alpha, long long n, c
                                              reinterpret_cast<__nv_bfloat162*>(y), alpha, n2);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // y[rows, Cpad] = [x[rows, C] | 0]: pads the latent's 4 channels to one 64-channel K chunk so the
@@ -193,7 +230,12 @@ __global__ void pad_channels_kernel(const __nv_bfloat16* __restrict__ x, __nv_bf
     reinterpret_cast<uint4*>(y)[i] = *reinterpret_cast<const uint4*>(v);
   }
 }
-int pad_channels(const void* x, void* y, int C, int Cpad, long long rows, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_pad_channels(const void* x, void* y, int32_t C, int32_t Cpad, int64_t rows, void* stream_ptr) {
+  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (C <= 0 || Cpad < C || (Cpad % 8) || rows <= 0) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(rows) * (Cpad / 8);
   int grid = static_cast<int>((total + 255) / 256);
@@ -202,6 +244,8 @@ int pad_channels(const void* x, void* y, int C, int Cpad, long long rows, cudaSt
                                                 reinterpret_cast<__nv_bfloat16*>(y), C, Cpad, static_cast<size_t>(rows));
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // SiLU on a small fp32/bf16 vector (embedding path), bf16 out
@@ -213,7 +257,12 @@ __global__ void silu_bf16_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloa
        i += static_cast<size_t>(gridDim.x) * blockDim.x)
     y[i] = __float2bfloat16(silu_f(__bfloat162float(x[i])));
 }
-int silu_bf16(const void* x, void* y, long long n, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_silu_bf16(const void* x, void* y, int64_t n, void* stream_ptr) {
+  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (n <= 0) return B200SR_EINVAL;
   int grid = static_cast<int>((n + 255) / 256);
   if (grid > num_sms() * 16) grid = num_sms() * 16;
@@ -221,6 +270,8 @@ int silu_bf16(const void* x, void* y, long long n, cudaStream_t stream) {
                                              reinterpret_cast<__nv_bfloat16*>(y), static_cast<size_t>(n));
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // sinusoidal embeddings: out[b, :] = cat(f(t*freq), g(t*freq)), freq_k = exp(-ln(max_period) k / half)
@@ -242,14 +293,21 @@ __global__ void sinusoid_kernel(const float* __restrict__ t, __nv_bfloat16* __re
   o[half + k] = __float2bfloat16(sin_first ? cs : sn);
   if ((dim & 1) && k == 0) o[dim - 1] = __float2bfloat16(0.f);
 }
-int sinusoid_embedding(const float* t, void* out, int B, int dim, float max_period, int sin_first,
-                       cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_sinusoid_embedding(const float* t, void* out, int32_t B, int32_t dim, float max_period,
+                                         int32_t sin_first, void* stream_ptr) {
+  if (t == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (B <= 0 || dim < 2) return B200SR_EINVAL;
   const int total = B * (dim / 2);
   launch_k(sinusoid_kernel, dim3((total + 127) / 128), dim3(128), 0, stream, 1, t, reinterpret_cast<__nv_bfloat16*>(out), B, dim, max_period,
                                                            sin_first);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // Direct 3x3 convolution (pad 1, stride 1) for tiny channel counts where an MMA tile would be
@@ -374,8 +432,13 @@ __global__ void conv3x3_few_out_kernel(const __nv_bfloat16* __restrict__ x, cons
   }
 }
 
-int conv3x3_small(const void* x, const void* w, const float* bias, const void* addend, void* y, int N, int H, int W,
-                  int Cin, int Cout, int out_nchw_f32, cudaStream_t stream) {
+}  // namespace b200sr
+
+extern "C" int b200sr_conv3x3_small(const void* x, const void* w, const float* bias, const void* addend, void* y,
+                                    int32_t N, int32_t H, int32_t W, int32_t Cin, int32_t Cout, int32_t out_nchw_f32,
+                                    void* stream_ptr) {
+  if (x == nullptr || w == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (N <= 0 || H <= 0 || W <= 0 || Cin <= 0 || Cout <= 0) return B200SR_EINVAL;
   const __nv_bfloat16* xi = reinterpret_cast<const __nv_bfloat16*>(x);
   const __nv_bfloat16* wi = reinterpret_cast<const __nv_bfloat16*>(w);
@@ -408,6 +471,8 @@ int conv3x3_small(const void* x, const void* w, const float* bias, const void* a
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
 
+namespace b200sr {
+
 // ------------------------------------------------------------------------------------------
 // Sampler step, part 1 (before the network):   sampling.py:598-606, denoiser.py:70-76, guiders.py:65-74
 //   x_hat = x + noise * s_noise * sqrt(sigma_hat^2 - sigma^2)          (fp32 NCHW, kept for part 2)
@@ -437,8 +502,13 @@ __global__ void sampler_pre_kernel(const float* __restrict__ x, const float* __r
       net_in[((static_cast<size_t>(k) * B + b) * HW + pix) * C + c] = o;
   }
 }
-int sampler_pre(const float* x, const float* noise, const float* scalars, float* x_hat, void* net_in, int B, int C,
-                int HW, int cfg_copies, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_sampler_pre(const float* x, const float* noise, const float* scalars, float* x_hat, void* net_in,
+                                  int32_t B, int32_t C, int32_t HW, int32_t cfg_copies, void* stream_ptr) {
+  if (x == nullptr || scalars == nullptr || x_hat == nullptr || net_in == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (B <= 0 || C <= 0 || HW <= 0 || cfg_copies < 1) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(B) * C * HW;
   int grid = static_cast<int>((total + 255) / 256);
@@ -447,6 +517,8 @@ int sampler_pre(const float* x, const float* noise, const float* scalars, float*
                                                HW, cfg_copies);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // Sampler step, part 2 (after the network):  denoiser.py:76-78, guiders.py:59-63, sampling.py:618-620
@@ -478,8 +550,13 @@ __global__ void sampler_post_kernel(const float* __restrict__ eps, const float* 
     x_next[i] = xh + d * (sigma_next - sigma_hat);
   }
 }
-int sampler_post(const float* eps, const float* x_hat, const float* scalars, float* denoised_out, float* x_next, int B,
-                 int C, int HW, int use_cfg, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_sampler_post(const float* eps, const float* x_hat, const float* scalars, float* denoised_out,
+                                   float* x_next, int32_t B, int32_t C, int32_t HW, int32_t use_cfg, void* stream_ptr) {
+  if (eps == nullptr || x_hat == nullptr || scalars == nullptr || x_next == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (B <= 0 || C <= 0 || HW <= 0) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(B) * C * HW;
   int grid = static_cast<int>((total + 255) / 256);
@@ -487,6 +564,8 @@ int sampler_post(const float* eps, const float* x_hat, const float* scalars, flo
   launch_k(sampler_post_kernel, dim3(grid), dim3(256), 0, stream, 1, eps, x_hat, scalars, denoised_out, x_next, B, C, HW, use_cfg);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // Euler update from an already guided `denoised` (cache-hit path reuses the previous one).
 __global__ void euler_from_denoised_kernel(const float* __restrict__ den, const float* __restrict__ x_hat,
@@ -501,14 +580,21 @@ __global__ void euler_from_denoised_kernel(const float* __restrict__ den, const 
     x_next[i] = xh + d * (sigma_next - sigma_hat);
   }
 }
-int euler_from_denoised(const float* denoised, const float* x_hat, const float* scalars, float* x_next, long long n,
-                        cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_euler_from_denoised(const float* denoised, const float* x_hat, const float* scalars, float* x_next,
+                                          int64_t n, void* stream_ptr) {
+  if (denoised == nullptr || x_hat == nullptr || scalars == nullptr || x_next == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (n <= 0) return B200SR_EINVAL;
   int grid = static_cast<int>((n + 255) / 256);
   if (grid > num_sms() * 8) grid = num_sms() * 8;
   launch_k(euler_from_denoised_kernel, dim3(grid), dim3(256), 0, stream, 1, denoised, x_hat, scalars, x_next, static_cast<size_t>(n));
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // Tile blend (sampling.py:753-756): acc[:, :, h0:h0+th, w0:w0+tw] += tile * weight ; cnt += weight
@@ -541,8 +627,14 @@ __global__ void tile_normalize_kernel(const float* __restrict__ acc, const float
        i += static_cast<size_t>(gridDim.x) * blockDim.x)
     out[i] = acc[i] / cnt[i];
 }
-int tile_accumulate(const float* tile, const float* weight, float* acc, float* cnt, int BC, int th, int tw, int H, int W,
-                    int h0, int w0, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_tile_accumulate(const float* tile, const float* weight, float* acc, float* cnt, int32_t BC,
+                                      int32_t th, int32_t tw, int32_t H, int32_t W, int32_t h0, int32_t w0,
+                                      void* stream_ptr) {
+  if (tile == nullptr || weight == nullptr || acc == nullptr) return B200SR_EINVAL;  // cnt may be NULL
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (BC <= 0 || th <= 0 || tw <= 0 || h0 < 0 || w0 < 0 || h0 + th > H || w0 + tw > W) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(BC) * th * tw;
   int grid = static_cast<int>((total + 255) / 256);
@@ -550,13 +642,17 @@ int tile_accumulate(const float* tile, const float* weight, float* acc, float* c
   launch_k(tile_accumulate_kernel, dim3(grid), dim3(256), 0, stream, 1, tile, weight, acc, cnt, BC, th, tw, H, W, h0, w0);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
-int tile_normalize(const float* acc, const float* cnt, float* out, long long n, cudaStream_t stream) {
+extern "C" int b200sr_tile_normalize(const float* acc, const float* cnt, float* out, int64_t n, void* stream_ptr) {
+  if (acc == nullptr || cnt == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (n <= 0) return B200SR_EINVAL;
   int grid = static_cast<int>((n + 255) / 256);
   if (grid > num_sms() * 8) grid = num_sms() * 8;
   launch_k(tile_normalize_kernel, dim3(grid), dim3(256), 0, stream, 1, acc, cnt, out, static_cast<size_t>(n));
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // First-block-cache similarity (DFBCache.py:98-112):
@@ -611,9 +707,16 @@ __global__ void rel_l1_finalize_kernel(double* __restrict__ sums, const float* _
   sums[0] = 0.0;
   sums[1] = 0.0;
 }
+
+}  // namespace b200sr
+
 // workspace: 2 doubles, zero on first use (re-zeroed by the finalize kernel)
-int rel_l1_similarity(const void* prev, const void* cur, long long n, const float* threshold, double* workspace,
-                      float* result, cudaStream_t stream) {
+extern "C" int b200sr_rel_l1_similarity(const void* prev, const void* cur, int64_t n, const float* threshold,
+                                        void* workspace_ptr, float* result, void* stream_ptr) {
+  if (prev == nullptr || cur == nullptr || threshold == nullptr || workspace_ptr == nullptr || result == nullptr)
+    return B200SR_EINVAL;
+  double* workspace = static_cast<double*>(workspace_ptr);
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (n <= 0 || (n % 8)) return B200SR_EINVAL;
   const size_t n8 = static_cast<size_t>(n) / 8;
   int grid = static_cast<int>((n8 + 255) / 256);
@@ -623,6 +726,8 @@ int rel_l1_similarity(const void* prev, const void* cur, long long n, const floa
   launch_k(rel_l1_finalize_kernel, dim3(1), dim3(1), 0, stream, 1, workspace, threshold, result, static_cast<double>(n));
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // SR3 ancestral DDPM update (diffusion.py:142-176), fp32 NCHW:
@@ -646,14 +751,21 @@ __global__ void sr3_update_kernel(const float* __restrict__ x, const float* __re
     out[i] = v;
   }
 }
-int sr3_update(const float* x, const float* eps, const float* noise, const float* scalars, float* out, long long n,
-               cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_sr3_update(const float* x, const float* eps, const float* noise, const float* scalars, float* out,
+                                 int64_t n, void* stream_ptr) {
+  if (x == nullptr || eps == nullptr || scalars == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (n <= 0) return B200SR_EINVAL;
   int grid = static_cast<int>((n + 255) / 256);
   if (grid > num_sms() * 8) grid = num_sms() * 8;
   launch_k(sr3_update_kernel, dim3(grid), dim3(256), 0, stream, 1, x, eps, noise, scalars, out, static_cast<size_t>(n));
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // Batched small device-to-device copies in ONE launch (per-step loader of the sampler engine: latent, noise,
@@ -683,18 +795,23 @@ __global__ void copy_batch_kernel(const CopyBatchArgs a) {
     for (size_t i = tid; i < static_cast<size_t>(nbytes >> 2); i += nth) dp[i] = sp[i];
   }
 }
-int copy_batch(const void* const* src, void* const* dst, const long long* bytes, int n, cudaStream_t stream) {
-  if (n <= 0 || n > B200SR_MAX_COPIES) return B200SR_EINVAL;
+
+}  // namespace b200sr
+
+extern "C" int b200sr_copy_batch(const b200sr_copy* copies, int32_t n, void* stream_ptr) {
+  if (copies == nullptr || n <= 0 || n > B200SR_MAX_COPIES) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   CopyBatchArgs a;
   long long mx = 0;
   for (int i = 0; i < n; ++i) {
-    if (src[i] == nullptr || dst[i] == nullptr || bytes[i] <= 0 || (bytes[i] & 3) ||
-        (reinterpret_cast<uintptr_t>(src[i]) & 3) || (reinterpret_cast<uintptr_t>(dst[i]) & 3))
+    const b200sr_copy& c = copies[i];
+    if (c.src == nullptr || c.dst == nullptr || c.bytes <= 0 || (c.bytes & 3) || (reinterpret_cast<uintptr_t>(c.src) & 3) ||
+        (reinterpret_cast<uintptr_t>(c.dst) & 3))
       return B200SR_EINVAL;
-    a.src[i] = src[i];
-    a.dst[i] = dst[i];
-    a.bytes[i] = bytes[i];
-    if (bytes[i] > mx) mx = bytes[i];
+    a.src[i] = c.src;
+    a.dst[i] = c.dst;
+    a.bytes[i] = c.bytes;
+    if (c.bytes > mx) mx = c.bytes;
   }
   int gx = static_cast<int>((mx / 16 + 255) / 256);
   if (gx < 1) gx = 1;
@@ -702,6 +819,8 @@ int copy_batch(const void* const* src, void* const* dst, const long long* bytes,
   launch_k(copy_batch_kernel, dim3(gx, n), dim3(256), 0, stream, 1, a);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // Tile-sharded blend, halo side (sampling.py:753-756 across GPUs): strip = tile[:, y0:y0+sh, x0:x0+sw] * weight
@@ -736,8 +855,13 @@ __global__ void strip_add_kernel(const float* __restrict__ strip, float* __restr
     acc[o] = __fadd_rn(acc[o], strip[i]);
   }
 }
-int tile_weighted_strip(const float* tile, const float* weight, float* strip, int BC, int th, int tw, int y0, int x0,
-                        int sh, int sw, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_tile_weighted_strip(const float* tile, const float* weight, float* strip, int32_t BC, int32_t th,
+                                          int32_t tw, int32_t y0, int32_t x0, int32_t sh, int32_t sw, void* stream_ptr) {
+  if (tile == nullptr || weight == nullptr || strip == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (BC <= 0 || sh <= 0 || sw <= 0 || y0 < 0 || x0 < 0 || y0 + sh > th || x0 + sw > tw) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(BC) * sh * sw;
   int grid = static_cast<int>((total + 255) / 256);
@@ -745,7 +869,10 @@ int tile_weighted_strip(const float* tile, const float* weight, float* strip, in
   launch_k(tile_weighted_strip_kernel, dim3(grid), dim3(256), 0, stream, 1, tile, weight, strip, BC, th, tw, y0, x0, sh, sw);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
-int strip_add(const float* strip, float* acc, int BC, int sh, int sw, int H, int W, int h0, int w0, cudaStream_t stream) {
+extern "C" int b200sr_strip_add(const float* strip, float* acc, int32_t BC, int32_t sh, int32_t sw, int32_t H, int32_t W,
+                                int32_t h0, int32_t w0, void* stream_ptr) {
+  if (strip == nullptr || acc == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (BC <= 0 || sh <= 0 || sw <= 0 || h0 < 0 || w0 < 0 || h0 + sh > H || w0 + sw > W) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(BC) * sh * sw;
   int grid = static_cast<int>((total + 255) / 256);
@@ -753,6 +880,8 @@ int strip_add(const float* strip, float* acc, int BC, int sh, int sw, int H, int
   launch_k(strip_add_kernel, dim3(grid), dim3(256), 0, stream, 1, strip, acc, BC, sh, sw, H, W, h0, w0);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // First-stage (SDXL VAE) glue around the latent: 1x1 convolutions between <= 8 channels
@@ -788,8 +917,13 @@ __global__ void pointwise_small_kernel(const __nv_bfloat16* __restrict__ x, cons
     }
   }
 }
-int pointwise_small(const void* x, const float* w, const float* bias, void* y, int Cin, int Cout, long long rows, int HW,
-                    int out_nchw_f32, float scale, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_pointwise_small(const void* x, const float* w, const float* bias, void* y, int32_t Cin, int32_t Cout,
+                                      int64_t rows, int32_t HW, int32_t out_nchw_f32, float scale, void* stream_ptr) {
+  if (x == nullptr || w == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (Cin <= 0 || Cin > 8 || Cout <= 0 || Cout > 8 || rows <= 0 || HW <= 0 || (rows % HW) != 0) return B200SR_EINVAL;
   int grid = static_cast<int>((rows + 255) / 256);
   if (grid > num_sms() * 16) grid = num_sms() * 16;
@@ -797,6 +931,8 @@ int pointwise_small(const void* x, const float* w, const float* bias, void* y, i
            Cout, rows, HW, out_nchw_f32, scale);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 __global__ void diag_gaussian_kernel(const float* __restrict__ moments, const float* __restrict__ noise,
                                      float* __restrict__ z, int C, int HW, long long total, float scale) {
@@ -814,8 +950,13 @@ __global__ void diag_gaussian_kernel(const float* __restrict__ moments, const fl
     z[i] = v * scale;
   }
 }
-int diag_gaussian(const float* moments, const float* noise, float* z, int N, int C, int HW, float scale,
-                  cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_diag_gaussian(const float* moments, const float* noise, float* z, int32_t N, int32_t C, int32_t HW,
+                                    float scale, void* stream_ptr) {
+  if (moments == nullptr || z == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (N <= 0 || C <= 0 || HW <= 0) return B200SR_EINVAL;
   const long long total = static_cast<long long>(N) * C * HW;
   int grid = static_cast<int>((total + 255) / 256);
@@ -823,6 +964,8 @@ int diag_gaussian(const float* moments, const float* noise, float* z, int N, int
   launch_k(diag_gaussian_kernel, dim3(grid), dim3(256), 0, stream, 1, moments, noise, z, C, HW, total, scale);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // Token + position embedding of the text towers (transformers CLIPTextEmbeddings; open_clip
@@ -844,15 +987,18 @@ __global__ void embed_tokens_kernel(const long long* __restrict__ ids, const flo
     out[i] = __float2bfloat16(tok[static_cast<size_t>(id) * C + c] + pos[static_cast<size_t>(t) * C + c]);
   }
 }
-int embed_tokens(const long long* ids, const float* tok, const float* pos, void* out, int B, int T, int C, int vocab,
-                 cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_embed_tokens(const int64_t* ids, const float* tok, const float* pos, void* out, int32_t B, int32_t T,
+                                   int32_t C, int32_t vocab, void* stream_ptr) {
+  if (ids == nullptr || tok == nullptr || pos == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (B <= 0 || T <= 0 || C <= 0 || vocab <= 0) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(B) * T * C;
   int grid = static_cast<int>((total + 255) / 256);
   if (grid > num_sms() * 8) grid = num_sms() * 8;
-  launch_k(embed_tokens_kernel, dim3(grid), dim3(256), 0, stream, 1, ids, tok, pos, reinterpret_cast<__nv_bfloat16*>(out), T, C,
+  launch_k(embed_tokens_kernel, dim3(grid), dim3(256), 0, stream, 1, reinterpret_cast<const long long*>(ids), tok, pos, reinterpret_cast<__nv_bfloat16*>(out), T, C,
            vocab, total);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
-
-}  // namespace b200sr

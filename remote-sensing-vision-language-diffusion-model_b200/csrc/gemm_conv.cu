@@ -1373,7 +1373,7 @@ static int launch_t(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtens
   return err == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
 
-static int fill_epilogue(GemmParams& p, const EpilogueArgs& e) {
+static int fill_epilogue(GemmParams& p, const b200sr_epilogue& e) {
   p.bias = e.bias;
   p.rowvec = e.rowvec;
   p.rows_per_group = e.rows_per_group;
@@ -1501,16 +1501,22 @@ static int finish(const CUtensorMap& tmA, const void* W, GemmParams& p, int real
   return cluster == 2 ? launch_t<2>(tmA, tmB, tmO, p, stream) : launch_t<1>(tmA, tmB, tmO, p, stream);
 }
 
-// The N tile gemm_bf16 picks for a plain GEMM (no softmax epilogue, force_bn = 0): a GEMM that writes row statistics
-// writes ceil(N / tile) partials per row, which the consuming GEMM has to be told.
-int gemm_n_tile(int M, int N, int K) {
+}  // namespace b200sr
+
+using namespace b200sr;
+
+// The N tile b200sr_gemm_bf16 picks for a plain GEMM (no softmax epilogue, force_bn = 0): a GEMM that writes row
+// statistics writes ceil(N / tile) partials per row, which the consuming GEMM has to be told.
+extern "C" int b200sr_gemm_n_tile(int32_t M, int32_t N, int32_t K) {
   if (M <= 0 || N <= 0 || K <= 0) return 0;
   const int m_blocks = (M + BLOCK_M - 1) / BLOCK_M;
   return pick_bn(m_blocks, N, (K + BLOCK_K - 1) / BLOCK_K, num_sms(), m_blocks >= 2 ? 2 : 1);
 }
 
-int gemm_bf16(const void* A, long long lda, const void* W, int M, int N, int K, const EpilogueArgs& e, int force_bn,
-              cudaStream_t stream) {
+extern "C" int b200sr_gemm_bf16(const void* A, int64_t lda, const void* W, int32_t M, int32_t N, int32_t K,
+                                const b200sr_epilogue* epi, int32_t force_bn, void* stream_ptr) {
+  if (A == nullptr || W == nullptr || epi == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (M <= 0 || N <= 0 || K <= 0 || (K % 8) != 0 || (lda % 8) != 0) return B200SR_EINVAL;
   GemmParams p{};
   p.mode = 0;
@@ -1518,7 +1524,7 @@ int gemm_bf16(const void* A, long long lda, const void* W, int M, int N, int K, 
   p.N = N;
   p.K = K;
   p.k_iters = (K + BLOCK_K - 1) / BLOCK_K;
-  int rc = fill_epilogue(p, e);
+  int rc = fill_epilogue(p, *epi);
   if (rc) return rc;
   CUtensorMap tmA;
   uint64_t dims[2] = {static_cast<uint64_t>(K), static_cast<uint64_t>(M)};
@@ -1530,13 +1536,16 @@ int gemm_bf16(const void* A, long long lda, const void* W, int M, int N, int K, 
 }
 
 // x: NHWC bf16 [NB, H, W, Cin]; w: [Cout, 3, 3, Cin] bf16 (K = tap*Cin + c); stride 1 or 2, pad 1.
-int conv3x3_bf16(const void* x, const void* w, int NB, int H, int W, int Cin, int Cout, int stride, int pad_lo,
-                 const EpilogueArgs& e, int force_bn, cudaStream_t stream) {
+extern "C" int b200sr_conv3x3_bf16(const void* x, const void* w, int32_t NB, int32_t H, int32_t W, int32_t Cin,
+                                   int32_t Cout, int32_t stride, int32_t pad_lo, const b200sr_epilogue* epi,
+                                   int32_t force_bn, void* stream_ptr) {
+  if (x == nullptr || w == nullptr || epi == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (NB <= 0 || H <= 0 || W <= 0 || Cin <= 0 || (Cin % BLOCK_K) != 0 || Cout <= 0) return B200SR_EINVAL;
   if (stride != 1 && stride != 2) return B200SR_EINVAL;
   if (pad_lo != 1 && !(pad_lo == 0 && stride == 2)) return B200SR_EINVAL;
   if (stride == 2 && ((H | W) & 1)) return B200SR_EINVAL;
-  if (e.geglu) return B200SR_EINVAL;
+  if (epi->geglu) return B200SR_EINVAL;
   const int OH = H / stride, OW = W / stride;
   // tile box: bw | OW, bw*bh*bn == 128, all powers of two
   int bw = 1;
@@ -1573,7 +1582,7 @@ int conv3x3_bf16(const void* x, const void* w, int NB, int H, int W, int Cin, in
   p.tiles_n = (NB + bn - 1) / bn;
   p.kc_per_tap = Cin / BLOCK_K;
   p.k_iters = 9 * p.kc_per_tap;
-  int rc = fill_epilogue(p, e);
+  int rc = fill_epilogue(p, *epi);
   if (rc) return rc;
   CUtensorMap tmA;
   if (stride == 1) {
@@ -1600,8 +1609,6 @@ int conv3x3_bf16(const void* x, const void* w, int NB, int H, int W, int Cin, in
   // Out-of-range spatial tiles (cluster round-up) decode to tn >= tiles_n: all rows masked, loads zero-filled.
   return finish(tmA, w, p, p.tiles_w * p.tiles_h * p.tiles_n, force_bn, stream);
 }
-
-}  // namespace b200sr
 
 #ifdef B200SR_GEMM_TRACE
 extern "C" void b200sr_debug_set_gemm_trace(void* p) { b200sr::g_gemm_trace = reinterpret_cast<long long*>(p); }

@@ -44,8 +44,15 @@ __global__ void wavelet_level_kernel(const float* __restrict__ img, float* __res
     if (high != nullptr) high[i] = (first ? 0.f : high[i]) + (r1[x] - l);
   }
 }
-int wavelet_level(const float* img, float* low, float* high, int first, int BC, int H, int W, int radius,
-                  cudaStream_t stream) {
+
+}  // namespace b200sr
+
+using namespace b200sr;
+
+extern "C" int b200sr_wavelet_level(const float* img, float* low, float* high, int32_t first, int32_t BC, int32_t H,
+                                    int32_t W, int32_t radius, void* stream_ptr) {
+  if (img == nullptr || low == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (BC <= 0 || H <= 0 || W <= 0 || radius <= 0 || img == low) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(BC) * H * W;
   int grid = static_cast<int>((total + 255) / 256);
@@ -53,6 +60,8 @@ int wavelet_level(const float* img, float* low, float* high, int first, int BC, 
   launch_k(wavelet_level_kernel, dim3(grid), dim3(256), 0, stream, 1, img, low, high, first, H, W, radius, total);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 __global__ void add_f32_kernel(const float* __restrict__ a, const float* __restrict__ b, float* __restrict__ out,
                                size_t n) {
@@ -62,13 +71,20 @@ __global__ void add_f32_kernel(const float* __restrict__ a, const float* __restr
        i += static_cast<size_t>(gridDim.x) * blockDim.x)
     out[i] = a[i] + b[i];
 }
-int add_f32(const float* a, const float* b, float* out, long long n, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_add_f32(const float* a, const float* b, float* out, int64_t n, void* stream_ptr) {
+  if (a == nullptr || b == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (n <= 0) return B200SR_EINVAL;
   int grid = static_cast<int>((n + 255) / 256);
   if (grid > num_sms() * 16) grid = num_sms() * 16;
   launch_k(add_f32_kernel, dim3(grid), dim3(256), 0, stream, 1, a, b, out, static_cast<size_t>(n));
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // cubic convolution coefficients of torch's upsample_bicubic2d (A = -0.75)
 __device__ __forceinline__ void cubic_coeffs(float t, float (&c)[4]) {
@@ -109,7 +125,13 @@ __global__ void image_to_u8_kernel(const float* __restrict__ x, uint8_t* __restr
     }
   }
 }
-int image_to_u8(const float* x, void* out, int C, int H, int W, int OH, int OW, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_image_to_u8(const float* x, void* out, int32_t C, int32_t H, int32_t W, int32_t OH, int32_t OW,
+                                  void* stream_ptr) {
+  if (x == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (C <= 0 || C > 4 || H <= 0 || W <= 0 || OH <= 0 || OW <= 0) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(OH) * OW;
   int grid = static_cast<int>((total + 255) / 256);
@@ -118,6 +140,8 @@ int image_to_u8(const float* x, void* out, int C, int H, int W, int OH, int OW, 
            static_cast<float>(H) / OH, static_cast<float>(W) / OW);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ---- stage-1 -> stage-2 hand-off (infer.py:133-138, models/util.py:132-156) -------------------------------------------
 static int grid_for(size_t work) {
@@ -155,7 +179,12 @@ __global__ void tensor2img_u8_kernel(const float* __restrict__ x, uint8_t* __res
     }
   }
 }
-int tensor2img_u8(const float* x, void* out, int C, int H, int W, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_tensor2img_u8(const float* x, void* out, int32_t C, int32_t H, int32_t W, void* stream_ptr) {
+  if (x == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (C <= 0 || C > 4 || H <= 0 || W <= 0) return B200SR_EINVAL;
   const size_t HW = static_cast<size_t>(H) * W;
   const bool vec = HW % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0;
@@ -163,6 +192,8 @@ int tensor2img_u8(const float* x, void* out, int C, int H, int W, cudaStream_t s
            reinterpret_cast<uint8_t*>(out), C, HW, vec);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // One axis of Pillow's 8-bit resample (libImaging/Resample.c ImagingResampleHorizontal_8bpc / ..Vertical_8bpc) over
 // src viewed as [outer, in_len, inner] bytes -> dst [outer, out_len, inner]: the horizontal pass of an HWC image is
@@ -206,8 +237,13 @@ __global__ void resample_u8_kernel(const uint8_t* __restrict__ src, uint8_t* __r
     }
   }
 }
-int resample_u8(const void* src, void* dst, int outer, int in_len, int out_len, int inner, const int* bounds,
-                const int* coeffs, int ksize, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_resample_u8(const void* src, void* dst, int32_t outer, int32_t in_len, int32_t out_len, int32_t inner,
+                                  const int32_t* bounds, const int32_t* coeffs, int32_t ksize, void* stream_ptr) {
+  if (src == nullptr || dst == nullptr || bounds == nullptr || coeffs == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (outer <= 0 || in_len <= 0 || out_len <= 0 || inner <= 0 || ksize <= 0 || src == dst) return B200SR_EINVAL;
   const size_t total = static_cast<size_t>(outer) * out_len * inner;
   const bool aligned = (reinterpret_cast<uintptr_t>(dst) & 15) == 0;
@@ -216,6 +252,8 @@ int resample_u8(const void* src, void* dst, int outer, int in_len, int out_len, 
            ksize, total, aligned);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // PIL2Tensor's conversion (models/util.py:152-154): x / 255 * 2 - 1 in float64, cast to fp32; uint8 HWC -> fp32 CHW.
 // Each thread converts 4 pixels and writes one 16-byte store per plane.
@@ -243,7 +281,12 @@ __global__ void img_u8_to_tensor_kernel(const uint8_t* __restrict__ in, float* _
     }
   }
 }
-int img_u8_to_tensor(const void* in, float* out, int C, int H, int W, cudaStream_t stream) {
+
+}  // namespace b200sr
+
+extern "C" int b200sr_img_u8_to_tensor(const void* in, float* out, int32_t C, int32_t H, int32_t W, void* stream_ptr) {
+  if (in == nullptr || out == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (C <= 0 || C > 4 || H <= 0 || W <= 0) return B200SR_EINVAL;
   const size_t HW = static_cast<size_t>(H) * W;
   const bool vec = HW % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0;
@@ -251,5 +294,3 @@ int img_u8_to_tensor(const void* in, float* out, int C, int H, int W, cudaStream
            reinterpret_cast<const uint8_t*>(in), out, C, HW, vec);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
-
-}  // namespace b200sr

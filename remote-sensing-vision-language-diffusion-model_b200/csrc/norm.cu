@@ -526,22 +526,32 @@ static bool gn_fused_eligible(int N, int C, int groups, int threads, int P, int 
   if (smem_out) *smem_out = smem;
   return gn_fused_enabled() && chunks * N <= num_sms() && N <= 128 && smem <= 100 * 1024 && fold_fits;
 }
-int group_norm_launches(int N, int HW, int C, int groups) {
+
+}  // namespace b200sr
+
+using namespace b200sr;
+
+extern "C" int b200sr_group_norm_launches(int32_t N, int32_t HW, int32_t C, int32_t groups) {
   if (N <= 0 || HW <= 0 || C <= 0 || groups <= 0 || (C % 8) != 0 || (C % groups) != 0) return 0;
   int threads, P, ppc, chunks;
   gn_geometry(N, HW, C, &threads, &P, &ppc, &chunks);
   return gn_fused_eligible(N, C, groups, threads, P, ppc, chunks, nullptr) ? 1 : 2;
 }
 
-size_t group_norm_workspace_bytes(int N, int HW, int C, int groups) {
+extern "C" size_t b200sr_group_norm_workspace_bytes(int32_t N, int32_t HW, int32_t C, int32_t groups) {
+  if (N <= 0 || HW <= 0 || C < 8 || groups <= 0) return 0;
   int threads, P, ppc, chunks;
   gn_geometry(N, HW, C, &threads, &P, &ppc, &chunks);
   return (GN_WS_COUNTER_FLOATS + 2 * static_cast<size_t>(N) * groups + static_cast<size_t>(N) * chunks * groups * 2) * sizeof(float);
 }
 
-int group_norm_nhwc(const void* x, void* y, const float* weight, const float* bias, int N, int HW, int C, int groups,
-                    float eps, int silu, const void* sft_gamma, const void* sft_beta, const void* raw,
-                    float control_scale, float* workspace, cudaStream_t stream) {
+extern "C" int b200sr_group_norm_nhwc(const void* x, void* y, const float* weight, const float* bias, int32_t N,
+                                      int32_t HW, int32_t C, int32_t groups, float eps, int32_t silu,
+                                      const void* sft_gamma, const void* sft_beta, const void* raw,
+                                      float control_scale, void* workspace_ptr, void* stream_ptr) {
+  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
+  float* workspace = static_cast<float*>(workspace_ptr);
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (N <= 0 || HW <= 0 || C <= 0 || groups <= 0 || (C % 8) != 0 || (C % groups) != 0 || C / 8 > 1024)
     return B200SR_EINVAL;
   if ((sft_gamma == nullptr) != (sft_beta == nullptr)) return B200SR_EINVAL;
@@ -597,8 +607,11 @@ int group_norm_nhwc(const void* x, void* y, const float* weight, const float* bi
 
 // Statistics pass alone: (mean, rstd) per (image, group) into `stats_out` [N][groups][2] for a consumer that applies
 // the normalisation itself (the halo convolution's fused input GroupNorm, gemm_conv.cu).
-int group_norm_stats(const void* x, int N, int HW, int C, int groups, float eps, float* stats_out, float* workspace,
-                     cudaStream_t stream) {
+extern "C" int b200sr_group_norm_stats(const void* x, int32_t N, int32_t HW, int32_t C, int32_t groups, float eps,
+                                       float* stats_out, void* workspace_ptr, void* stream_ptr) {
+  if (x == nullptr) return B200SR_EINVAL;
+  float* workspace = static_cast<float*>(workspace_ptr);
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (N <= 0 || HW <= 0 || C <= 0 || groups <= 0 || (C % 8) != 0 || (C % groups) != 0 || C / 8 > 1024)
     return B200SR_EINVAL;
   if (workspace == nullptr || stats_out == nullptr || N > GN_WS_COUNTER_FLOATS) return B200SR_EINVAL;
@@ -609,6 +622,8 @@ int group_norm_stats(const void* x, int N, int HW, int C, int groups, float eps,
            chunks, N, eps);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // LayerNorm over the channel dim of a token-major [M, C] bf16 matrix: one warp per row, the row
@@ -683,8 +698,12 @@ layer_norm_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict
   }
 }
 
-int layer_norm(const void* x, void* y, const float* weight, const float* bias, int M, int C, float eps,
-               cudaStream_t stream) {
+}  // namespace b200sr
+
+extern "C" int b200sr_layer_norm(const void* x, void* y, const float* weight, const float* bias, int32_t M, int32_t C,
+                                 float eps, void* stream_ptr) {
+  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (M <= 0 || C <= 0 || (C % 8) != 0 || C > 2560 * 2 || weight == nullptr || bias == nullptr) return B200SR_EINVAL;
   const int rows_per_cta = 8;
   const int grid = (M + rows_per_cta - 1) / rows_per_cta;
@@ -703,6 +722,8 @@ int layer_norm(const void* x, void* y, const float* weight, const float* bias, i
     launch_k(layer_norm_kernel<20>, dim3(grid), dim3(256), 0, stream, 1, xi, yo, weight, bias, M, C, eps);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
+
+namespace b200sr {
 
 // ------------------------------------------------------------------------------------------
 // Row softmax of an fp32 [rows, cols] score matrix -> bf16 probabilities (SR3 single-head
@@ -803,8 +824,12 @@ __global__ void __launch_bounds__(256) row_softmax_fold_kernel(const float2* __r
   pdl_launch_dependents();
 }
 
-int row_softmax_fold(const float* parts, int n_parts, long long rows, float* out, cudaStream_t stream) {
+}  // namespace b200sr
+
+extern "C" int b200sr_row_softmax_fold(const float* parts, int32_t n_parts, int64_t rows, float* out,
+                                       void* stream_ptr) {
   if (parts == nullptr || out == nullptr || n_parts <= 0 || rows <= 0) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   const unsigned grid = static_cast<unsigned>((rows + 255) / 256);
   return launch_k(row_softmax_fold_kernel, dim3(grid), dim3(256), 0, stream, 1, reinterpret_cast<const float2*>(parts), n_parts,
                   rows, reinterpret_cast<float2*>(out)) == cudaSuccess
@@ -812,7 +837,10 @@ int row_softmax_fold(const float* parts, int n_parts, long long rows, float* out
              : B200SR_ELAUNCH;
 }
 
-int softmax_rows(const float* x, void* y, int rows, int cols, int valid, float scale, cudaStream_t stream) {
+extern "C" int b200sr_softmax_rows(const float* x, void* y, int32_t rows, int32_t cols, int32_t valid, float scale,
+                                   void* stream_ptr) {
+  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
+  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
   if (rows <= 0 || cols <= 0 || valid <= 0 || valid > cols) return B200SR_EINVAL;
   if (cols > 1024 && cols <= 32768 && (cols % 4) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
       (reinterpret_cast<uintptr_t>(y) & 7) == 0) {
@@ -830,5 +858,3 @@ int softmax_rows(const float* x, void* y, int rows, int cols, int valid, float s
              ? B200SR_OK
              : B200SR_ELAUNCH;
 }
-
-}  // namespace b200sr
