@@ -110,7 +110,9 @@ typedef struct b200sr_epilogue {
  * Replaces nn.Linear / 1x1 nn.Conv2d: sgm/modules/attention.py:213-218 (to_q/k/v, to_out),
  * :84-91 (GEGLU), :106 (FF out), :587/:611 (proj_in/out); openaimodel.py:283-287 (emb_layers),
  * :311 (skip 1x1), :657-691 (time_embed/label_emb); SR_modules.py:84 (zero_conv).
- * lda in elements; K % 8 == 0; N % 8 == 0; force_bn = 0 lets the library pick the N tile.    */
+ * lda in elements; K % 8 == 0; N % 8 == 0; force_bn = 0 lets the library pick the N tile.
+ * Both this and b200sr_conv3x3_bf16: out, residual and rowvec 16-byte aligned, ln_stats / ln_stats_out 8-byte
+ * aligned, ldc >= the output width, ldr >= N; EINVAL otherwise.                                 */
 int b200sr_gemm_bf16(const void* A, int64_t lda, const void* W, int32_t M, int32_t N, int32_t K,
                      const b200sr_epilogue* epi, int32_t force_bn, void* stream);
 

@@ -1404,6 +1404,12 @@ static int fill_epilogue(GemmParams& p, const b200sr_epilogue& e) {
   p.ln_stats_out = reinterpret_cast<float2*>(e.ln_stats_out);
   p.row_softmax = e.row_softmax;
   p.row_softmax_valid = e.row_softmax_valid > 0 ? e.row_softmax_valid : p.N;
+  // The epilogue moves out, residual and rowvec in 16-byte vectors (uint4 / float4) from row starts that the ld checks
+  // keep 16-byte aligned relative to the base, and the row statistics in 8-byte float2 pairs.
+  const auto misaligned = [](const void* ptr, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(ptr) & (bytes - 1)) != 0; };
+  if (misaligned(e.out, 16) || misaligned(e.residual, 16) || misaligned(e.rowvec, 16) || misaligned(e.ln_stats, 8) ||
+      misaligned(e.ln_stats_out, 8))
+    return B200SR_EINVAL;
   if (e.row_softmax != 0) {
     // two-pass row softmax: plain GEMM, no other epilogue term; pass 1 writes statistics only, pass 2 bf16 probabilities
     if (p.mode != 0 || e.row_softmax < 0 || e.row_softmax > 2 || e.geglu || e.out_fp32 || e.residual != nullptr ||
@@ -1413,7 +1419,7 @@ static int fill_epilogue(GemmParams& p, const b200sr_epilogue& e) {
     if (e.row_softmax == 1 && (e.ln_stats_out == nullptr || e.ln_stats != nullptr)) return B200SR_EINVAL;
     if (e.row_softmax == 2 && (e.ln_stats == nullptr || e.ln_parts <= 0 || e.ln_stats_out != nullptr || e.out == nullptr))
       return B200SR_EINVAL;
-    if ((p.N % 8) != 0 || (e.row_softmax == 2 && (e.ldc % 8) != 0)) return B200SR_EINVAL;
+    if ((p.N % 8) != 0 || (e.row_softmax == 2 && ((e.ldc % 8) != 0 || e.ldc < p.N))) return B200SR_EINVAL;
     p.out = e.out;
     p.ldc = e.ldc;
     p.alpha = e.alpha;
@@ -1444,6 +1450,8 @@ static int fill_epilogue(GemmParams& p, const b200sr_epilogue& e) {
   if (e.geglu && (e.out_fp32 || e.residual != nullptr || e.rowvec != nullptr || (p.N % 32) != 0)) return B200SR_EINVAL;
   if (p.N % 8 != 0) return B200SR_EINVAL;
   if ((e.ldc % 8) != 0 || (e.residual != nullptr && (e.ldr % 8) != 0)) return B200SR_EINVAL;
+  // rows must not overlap: out has N (GEGLU: N / 2) columns, the residual N
+  if (e.ldc < (e.geglu ? p.N / 2 : p.N) || (e.residual != nullptr && e.ldr < p.N)) return B200SR_EINVAL;
   return B200SR_OK;
 }
 
