@@ -27,7 +27,7 @@ extern "C" {
 #endif
 
 /* Library / device introspection. */
-#define B200SR_ABI_VERSION 7  /* what b200sr_abi_version() returns */
+#define B200SR_ABI_VERSION 8  /* what b200sr_abi_version() returns */
 int b200sr_abi_version(void);         /* bumps on any signature change */
 int b200sr_num_sms(void);             /* SM count of the current device, <0 on error */
 
@@ -131,13 +131,6 @@ int b200sr_gemm_n_tile(int32_t M, int32_t N, int32_t K);
 int b200sr_conv3x3_bf16(const void* x, const void* w, int32_t N, int32_t H, int32_t W, int32_t Cin, int32_t Cout,
                         int32_t stride, int32_t pad_lo, const b200sr_epilogue* epi, int32_t force_bn, void* stream);
 
-/* Direct 3x3 convolution (pad 1, stride 1) for tiny channel counts: Cin <= 8 (Cout % 8 == 0),
- * or Cout <= 4 (Cin % 8 == 0).  `addend` (bf16 NHWC, few-in only) is added to the result
- * (GLVControl `h += guided_hint`, SR_modules.py:521-531).  out_nchw_f32 (few-out only) writes
- * fp32 NCHW (UNet `out`, openaimodel.py:941-947; wrappers.py:110 `.float()`).                 */
-int b200sr_conv3x3_small(const void* x, const void* w, const float* bias, const void* addend, void* y, int32_t N,
-                         int32_t H, int32_t W, int32_t Cin, int32_t Cout, int32_t out_nchw_f32, void* stream);
-
 /* GroupNorm over NHWC bf16 with optional fused SiLU and ZeroSFT modulation:
  *   y = GN(x) * w + b ; [SiLU] ; [y = y * (1 + gamma) + beta ; y = y*s + raw*(1-s)]
  * util.py:258-276, attention.py:122-125, openaimodel.py:254-258; SR_modules.py:101-110.
@@ -180,16 +173,9 @@ int b200sr_attention_d64(const void* q, int64_t ldq, int32_t q_col, const void* 
  * (M, L) pair per row, out [rows, 2]; pass 2 then takes ln_stats = out, ln_parts = 1.                             */
 int b200sr_row_softmax_fold(const float* parts, int32_t n_parts, int64_t rows, float* out, void* stream);
 
-/* y = softmax(x * scale) over the first valid_cols entries of each row (the rest are written as 0: zero-
- * padded keys); x fp32 [rows, cols], y bf16.  SR3 SelfAttention (one head of width C, scores from
- * b200sr_gemm_bf16 with fp32 output): models/sr3_model/sr3_modules/unet.py:133-138. */
-int b200sr_softmax_rows(const float* x, void* y, int32_t rows, int32_t cols, int32_t valid_cols, float scale,
-                        void* stream);
-
 /* Layout conversion at the nn.Module boundary. */
 int b200sr_nchw_f32_to_nhwc_bf16(const float* x, void* y, int32_t N, int32_t C, int32_t HW, float scale, void* stream);
-int b200sr_nhwc_bf16_to_nchw_f32(const void* x, float* y, int32_t N, int32_t C, int32_t HW, void* stream);
-/* same, from a source with Cs >= C channels per pixel (the first C are converted): the result of a convolution to <= 4
+/* bf16 NHWC -> fp32 NCHW from Cs >= C channels per pixel (the first C are converted): the result of a convolution to <= 4
  * channels that ran on the tensor cores with its output padded to 8 (UNet `out` openaimodel.py:941-947 + wrappers.py:110
  * `.float()`; SR3 final_conv; the first stage's decoder conv_out). */
 int b200sr_nhwc_bf16_to_nchw_f32_strided(const void* x, float* y, int32_t N, int32_t C, int32_t Cs, int32_t HW, void* stream);

@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # B200SR_LIB selects another in-tree build of the same ABI (A/B kernel experiments); default = the product library
 LIB_PATH = os.path.join(_HERE, os.environ.get("B200SR_LIB", "libb200sr.so"))
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 c_void_p, c_int, c_i64, c_float, c_size_t = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
 
@@ -86,7 +86,6 @@ SIGNATURES = {
     "b200sr_conv3x3_bf16": (c_int, [P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, C.POINTER(Epilogue), c_int, P]),
     "b200sr_pointwise_small": (c_int, [P, P, P, P, c_int, c_int, c_i64, c_int, c_int, c_float, P]),
     "b200sr_diag_gaussian": (c_int, [P, P, P, c_int, c_int, c_int, c_float, P]),
-    "b200sr_conv3x3_small": (c_int, [P, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, P]),
     "b200sr_group_norm_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
     "b200sr_group_norm_launches": (c_int, [c_int, c_int, c_int, c_int]),
     "b200sr_group_norm_nhwc": (
@@ -100,9 +99,7 @@ SIGNATURES = {
         [P, c_i64, c_int, P, c_i64, c_int, P, c_i64, c_int, P, c_i64, c_int, c_int, c_int, c_int, c_float, c_int, P, P],
     ),
     "b200sr_attention_d64_workspace_bytes": (C.c_size_t, [c_int, c_int, c_int, c_int]),
-    "b200sr_softmax_rows": (c_int, [P, P, c_int, c_int, c_int, c_float, P]),
     "b200sr_nchw_f32_to_nhwc_bf16": (c_int, [P, P, c_int, c_int, c_int, c_float, P]),
-    "b200sr_nhwc_bf16_to_nchw_f32": (c_int, [P, P, c_int, c_int, c_int, P]),
     "b200sr_nhwc_bf16_to_nchw_f32_strided": (c_int, [P, P, c_int, c_int, c_int, c_int, P]),
     "b200sr_upsample2x_nhwc": (c_int, [P, P, c_int, c_int, c_int, c_int, P]),
     "b200sr_concat_add": (c_int, [P, c_int, P, c_int, P, P, c_i64, P]),

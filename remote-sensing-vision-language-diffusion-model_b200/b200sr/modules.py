@@ -23,7 +23,6 @@ accumulation, fp32 normalisation statistics and softmax; activations are stored 
 """
 from __future__ import annotations
 
-import os
 from typing import Dict, List, Optional
 
 import torch
@@ -173,19 +172,13 @@ def _conv3x3(holder: Packed, name: str, conv: nn.Conv2d, x_nhwc: torch.Tensor, *
     return ops.conv3x3(x_nhwc, w, b, **kw)
 
 
-# LayerNorm folded around the GEMM behind it (transformer blocks): statistics ride from each residual GEMM's epilogue to the
-# next GEMM's epilogue, no LayerNorm kernel and no normalised copy of the residual stream (ops.gemm `ln` / `want_stats`)
-FUSE_LN_INTO_GEMM = os.environ.get("B200SR_FUSE_LN", "1") != "0"
-FUSE_GN_INTO_CONV = True   # GroupNorm + SiLU applied to the convolution's staged input tiles instead of a pass through HBM
-
-
 def _gn_silu_conv3x3(holder: Packed, name: str, norm: nn.GroupNorm, conv: nn.Conv2d, x_nhwc: torch.Tensor, **kw) -> torch.Tensor:
     """conv3x3(SiLU(GroupNorm(x))) (openaimodel.py:254-258, :289-300; model.py:127-141; sr3 unet.py:81-92).  Where the
     halo-path convolution applies (stride 1, W % 8 == 0, H >= 16) and the output fits one N tile (<= 256 channels: the
     high-resolution levels of SR3 and of the first stage) only the statistics pass runs as a kernel of its own: the
     convolution normalises its input tiles in shared memory.  Same arithmetic, same bf16 rounding point, so the result
     equals the two-kernel form bit for bit."""
-    if FUSE_GN_INTO_CONV and ops.conv3x3_gn_fusable(x_nhwc, 1, conv.out_channels) and norm.affine:
+    if ops.conv3x3_gn_fusable(x_nhwc, 1, conv.out_channels) and norm.affine:
         stats = ops.group_norm_stats(x_nhwc, norm.num_groups, norm.eps)
         return _conv3x3(holder, name, conv, x_nhwc, gn=(stats, norm.weight, norm.bias, norm.num_groups, True), **kw)
     return _conv3x3(holder, name, conv, _gn(norm, x_nhwc, silu=True), **kw)
@@ -364,9 +357,9 @@ class CrossAttention(nn.Module, Packed):
         return self._pk("kv", (self.to_k.weight, self.to_v.weight), lambda k, v: torch.cat([k, v], 0).to(bf16).contiguous())
 
     def _fold_norm(self) -> Optional[nn.LayerNorm]:
-        """The LayerNorm in front of this attention (set by BasicTransformerBlock) when it is to be folded into the
-        bound keys, else None."""
-        return self.__dict__.get("_pre_norm") if FUSE_LN_INTO_GEMM else None
+        """The LayerNorm in front of this attention (set by BasicTransformerBlock), folded into the bound keys; None
+        when there is none."""
+        return self.__dict__.get("_pre_norm")
 
     def _weights_key(self):
         ps = [self.to_q.weight, self.to_k.weight, self.to_v.weight, self.to_out[0].weight]
@@ -565,15 +558,10 @@ class SpatialTransformer(nn.Module, Packed):
         context = [tokens_bf16(c) if c is not None else None for c in context]
         b, h, w, c = x.shape
         t = _gn(self.norm, x).view(b, h * w, c)
-        stats = None
-        if FUSE_LN_INTO_GEMM:
-            t, stats = _linear(self, "proj_in", self.proj_in, t, want_stats=True)
-        else:
-            t = _linear(self, "proj_in", self.proj_in, t)
+        t, stats = _linear(self, "proj_in", self.proj_in, t, want_stats=True)
         last = len(self.transformer_blocks) - 1
         for i, block in enumerate(self.transformer_blocks):
-            r = block(t, context=context[i if len(context) > 1 else 0], stats=stats,
-                      want_stats=stats is not None and i < last)
+            r = block(t, context=context[i if len(context) > 1 else 0], stats=stats, want_stats=i < last)
             t, stats = r if isinstance(r, tuple) else (r, None)
         t = _linear(self, "proj_out", self.proj_out, t, residual=x.view(b, h * w, c))
         return t.view(b, h, w, c)

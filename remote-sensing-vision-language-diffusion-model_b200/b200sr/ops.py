@@ -352,30 +352,6 @@ def conv3x3(
     return out
 
 
-def conv3x3_small(
-    x: torch.Tensor,
-    w: torch.Tensor,
-    bias: Optional[torch.Tensor],
-    *,
-    addend: Optional[torch.Tensor] = None,
-    out_nchw_f32: bool = False,
-) -> torch.Tensor:
-    _req(x, bf16, "conv3x3_small.x")
-    _req(w, bf16, "conv3x3_small.w")
-    n, h, wd, cin = x.shape
-    cout = w.shape[0]
-    if out_nchw_f32:
-        out = torch.empty(n, cout, h, wd, dtype=torch.float32, device=x.device)
-    else:
-        out = torch.empty(n, h, wd, cout, dtype=bf16, device=x.device)
-    rc = _lib.load().b200sr_conv3x3_small(
-        x.data_ptr(), w.data_ptr(), _ptr(bias), _ptr(addend), out.data_ptr(), n, h, wd, cin, cout, int(out_nchw_f32),
-        _stream()
-    )
-    check(rc, f"conv3x3_small Cin={cin} Cout={cout}")
-    return out
-
-
 # ------------------------------------------------------------------------------------------------
 # normalisation
 # ------------------------------------------------------------------------------------------------
@@ -473,18 +449,7 @@ def attention(
     return out
 
 
-def softmax_rows(x: torch.Tensor, scale: float = 1.0, valid_cols: Optional[int] = None) -> torch.Tensor:
-    """softmax(x * scale) over the first `valid_cols` columns (others -> 0): fp32 [..., cols] -> bf16."""
-    _req(x, torch.float32, "softmax_rows.x")
-    cols = x.shape[-1]
-    y = torch.empty(x.shape, dtype=bf16, device=x.device)
-    check(_lib.load().b200sr_softmax_rows(x.data_ptr(), y.data_ptr(), x.numel() // cols, cols,
-                                          cols if valid_cols is None else valid_cols, float(scale), _stream()),
-          "softmax_rows")
-    return y
-
-
-SCORE_CHUNK_BYTES = 1 << 30   # fp32 score rows held at once by single_head_attention (T = 16384: the whole 1 GB matrix)
+SCORE_CHUNK_BYTES = 1 << 30   # bf16 probability rows held at once by single_head_attention (T = 16384: the whole 512 MB matrix)
 
 
 def gemm_row_softmax(a: torch.Tensor, w: torch.Tensor, scale: float, valid_cols: Optional[int] = None,
@@ -519,9 +484,6 @@ def gemm_row_softmax(a: torch.Tensor, w: torch.Tensor, scale: float, valid_cols:
     return out
 
 
-TWO_PASS_SOFTMAX = True   # single_head_attention: scores recomputed instead of stored (False: score GEMM -> softmax_rows)
-
-
 def single_head_attention(q: torch.Tensor, k: torch.Tensor, v_t: torch.Tensor, scale: float,
                           out_bias: Optional[torch.Tensor] = None, valid_keys: Optional[int] = None) -> torch.Tensor:
     """softmax(q k^T * scale) v for ONE head of width C = 512 (SR3 SelfAttention, sr3_modules/unet.py:114-143; the
@@ -529,21 +491,16 @@ def single_head_attention(q: torch.Tensor, k: torch.Tensor, v_t: torch.Tensor, s
     (V transposed = the B operand of P V); returns [T, C] bf16 (+ out_bias[C]).
 
     The output accumulator of a 128-row tile at C = 512 fills all 512 TMEM columns, which leaves no room for the score
-    tile, so this shape runs as score GEMM -> row softmax -> P V GEMM over query chunks sized to keep the fp32 scores
-    within SCORE_CHUNK_BYTES (never the T x T matrix: 17 GB at T = 65536)."""
+    tile, so this shape runs as gemm_row_softmax (two passes of the score GEMM) -> P V GEMM over query chunks sized to
+    keep the bf16 probabilities within SCORE_CHUNK_BYTES (never the T x T matrix: 8.6 GB at T = 65536)."""
     t, c = q.shape
     tk = k.shape[0]
-    two_pass = TWO_PASS_SOFTMAX and tk % 8 == 0
-    rows = (SCORE_CHUNK_BYTES // ((2 if two_pass else 4) * tk)) // 256 * 256
+    rows = (SCORE_CHUNK_BYTES // (2 * tk)) // 256 * 256
     rows = max(256, min(rows, t))
     out = torch.empty(t, c, dtype=bf16, device=q.device)
     for r0 in range(0, t, rows):
         r1 = min(t, r0 + rows)
-        if two_pass:
-            p = gemm_row_softmax(q[r0:r1], k, scale, valid_keys)                    # [rows, Tk] bf16 probabilities
-        else:
-            s = gemm(q[r0:r1], k, out_fp32=True, w_dynamic=True)                    # [rows, Tk] fp32 scores
-            p = softmax_rows(s, scale, valid_cols=valid_keys)
+        p = gemm_row_softmax(q[r0:r1], k, scale, valid_keys)                        # [rows, Tk] bf16 probabilities
         gemm(p, v_t, out_bias, w_dynamic=True, out=out[r0:r1])
     return out
 
@@ -569,14 +526,6 @@ def cast_bf16(x: torch.Tensor) -> torch.Tensor:
     y = torch.empty(x.shape, dtype=bf16, device=x.device)
     check(_lib.load().b200sr_nchw_f32_to_nhwc_bf16(x.data_ptr(), y.data_ptr(), 1, 1, x.numel(), 1.0, _stream()),
           "cast_bf16")
-    return y
-
-
-def nhwc_to_nchw_f32(x: torch.Tensor) -> torch.Tensor:
-    _req(x, bf16, "nhwc_to_nchw.x")
-    n, h, w, c = x.shape
-    y = torch.empty(n, c, h, w, dtype=torch.float32, device=x.device)
-    check(_lib.load().b200sr_nhwc_bf16_to_nchw_f32(x.data_ptr(), y.data_ptr(), n, c, h * w, _stream()), "nhwc_to_nchw")
     return y
 
 

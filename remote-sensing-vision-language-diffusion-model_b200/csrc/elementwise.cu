@@ -85,9 +85,6 @@ extern "C" int b200sr_nhwc_bf16_to_nchw_f32_strided(const void* x, float* y, int
   launch_k(nhwc_bf16_to_nchw_f32_kernel, dim3(grid), dim3(block), 0, stream, 1, reinterpret_cast<const __nv_bfloat16*>(x), y, C, Cs, HW);
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
-extern "C" int b200sr_nhwc_bf16_to_nchw_f32(const void* x, float* y, int32_t N, int32_t C, int32_t HW, void* stream) {
-  return b200sr_nhwc_bf16_to_nchw_f32_strided(x, y, N, C, C, HW, stream);
-}
 
 namespace b200sr {
 
@@ -304,170 +301,6 @@ extern "C" int b200sr_sinusoid_embedding(const float* t, void* out, int32_t B, i
   const int total = B * (dim / 2);
   launch_k(sinusoid_kernel, dim3((total + 127) / 128), dim3(128), 0, stream, 1, t, reinterpret_cast<__nv_bfloat16*>(out), B, dim, max_period,
                                                            sin_first);
-  return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
-}
-
-namespace b200sr {
-
-// ------------------------------------------------------------------------------------------
-// Direct 3x3 convolution (pad 1, stride 1) for tiny channel counts where an MMA tile would be
-// >90 % padding: Cin <= 8 (latent / image -> features) or Cout <= 8 (features -> latent / image).
-// NHWC bf16 in, weights [Cout, 3, 3, Cin] bf16, bias fp32.  Output bf16 NHWC, or fp32 NCHW when
-// out_nchw_f32 (the UNet `out` conv feeds the fp32 sampler directly).
-// ------------------------------------------------------------------------------------------
-__global__ void conv3x3_few_in_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ w,
-                                      const float* __restrict__ bias, const __nv_bfloat16* __restrict__ addend,
-                                      __nv_bfloat16* __restrict__ y, int N, int H, int W, int Cin, int Cout) {
-  pdl_launch_dependents();
-  pdl_wait();
-  // one thread = one output pixel x 8 output channels; weights staged in smem as fp32
-  extern __shared__ float s_w[];  // [Cout][9*Cin]
-  const int K = 9 * Cin;
-  for (int i = threadIdx.x; i < Cout * K; i += blockDim.x) s_w[i] = __bfloat162float(w[i]);
-  __syncthreads();
-  const int Co8 = Cout / 8;
-  const size_t total = static_cast<size_t>(N) * H * W * Co8;
-  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < total;
-       i += static_cast<size_t>(gridDim.x) * blockDim.x) {
-    const int cg = static_cast<int>(i % Co8);
-    size_t t = i / Co8;
-    const int ow = static_cast<int>(t % W);
-    t /= W;
-    const int oh = static_cast<int>(t % H);
-    const size_t n = t / H;
-    float acc[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[j] = bias ? bias[cg * 8 + j] : 0.f;
-    for (int kh = 0; kh < 3; ++kh) {
-      const int ih = oh + kh - 1;
-      if (ih < 0 || ih >= H) continue;
-      for (int kw = 0; kw < 3; ++kw) {
-        const int iw = ow + kw - 1;
-        if (iw < 0 || iw >= W) continue;
-        const __nv_bfloat16* px = x + ((n * H + ih) * W + iw) * Cin;
-        for (int c = 0; c < Cin; ++c) {
-          const float xv = __bfloat162float(px[c]);
-          const int kidx = (kh * 3 + kw) * Cin + c;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) acc[j] += xv * s_w[(cg * 8 + j) * K + kidx];
-        }
-      }
-    }
-    const size_t o = (((n * H + oh) * W + ow) * Cout) + cg * 8;
-    if (addend != nullptr) {
-      const uint4 u = __ldg(reinterpret_cast<const uint4*>(addend + o));
-      const uint32_t uu[4] = {u.x, u.y, u.z, u.w};
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float2 f = unpack_bf16x2(uu[j]);
-        acc[2 * j] += f.x;
-        acc[2 * j + 1] += f.y;
-      }
-    }
-    uint4 v;
-    v.x = pack_bf16x2(acc[0], acc[1]);
-    v.y = pack_bf16x2(acc[2], acc[3]);
-    v.z = pack_bf16x2(acc[4], acc[5]);
-    v.w = pack_bf16x2(acc[6], acc[7]);
-    *reinterpret_cast<uint4*>(y + o) = v;
-  }
-}
-
-template <int COUT>
-__global__ void conv3x3_few_out_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ w,
-                                       const float* __restrict__ bias, void* __restrict__ y, int N, int H, int W,
-                                       int Cin, int out_nchw_f32) {
-  pdl_launch_dependents();
-  pdl_wait();
-  // one warp = one output pixel; lanes stride over (tap, channel-vector); warp-shuffle reduction
-  const int warps_per_cta = blockDim.x >> 5;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int C8 = Cin / 8;
-  const size_t total = static_cast<size_t>(N) * H * W;
-  for (size_t pix = blockIdx.x * static_cast<size_t>(warps_per_cta) + warp; pix < total;
-       pix += static_cast<size_t>(gridDim.x) * warps_per_cta) {
-    const int ow = static_cast<int>(pix % W);
-    const int oh = static_cast<int>((pix / W) % H);
-    const size_t n = pix / (static_cast<size_t>(W) * H);
-    float acc[COUT];
-#pragma unroll
-    for (int j = 0; j < COUT; ++j) acc[j] = 0.f;
-    for (int idx = lane; idx < 9 * C8; idx += 32) {
-      const int tap = idx / C8, cv = idx - tap * C8;
-      const int kh = tap / 3, kw = tap - kh * 3;
-      const int ih = oh + kh - 1, iw = ow + kw - 1;
-      if (ih < 0 || ih >= H || iw < 0 || iw >= W) continue;
-      const uint4 u = __ldg(reinterpret_cast<const uint4*>(x + ((n * H + ih) * W + iw) * Cin) + cv);
-      const uint32_t uu[4] = {u.x, u.y, u.z, u.w};
-      float xv[8];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float2 f = unpack_bf16x2(uu[j]);
-        xv[2 * j] = f.x;
-        xv[2 * j + 1] = f.y;
-      }
-#pragma unroll
-      for (int co = 0; co < COUT; ++co) {
-        const uint4 wv = __ldg(reinterpret_cast<const uint4*>(w + (static_cast<size_t>(co) * 9 + tap) * Cin) + cv);
-        const uint32_t ww[4] = {wv.x, wv.y, wv.z, wv.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float2 f = unpack_bf16x2(ww[j]);
-          acc[co] += xv[2 * j] * f.x + xv[2 * j + 1] * f.y;
-        }
-      }
-    }
-#pragma unroll
-    for (int co = 0; co < COUT; ++co) acc[co] = warp_sum(acc[co]);
-    if (lane == 0) {
-#pragma unroll
-      for (int co = 0; co < COUT; ++co) {
-        const float v = acc[co] + (bias ? bias[co] : 0.f);
-        if (out_nchw_f32)
-          reinterpret_cast<float*>(y)[((n * COUT + co) * H + oh) * W + ow] = v;
-        else
-          reinterpret_cast<__nv_bfloat16*>(y)[pix * COUT + co] = __float2bfloat16(v);
-      }
-    }
-  }
-}
-
-}  // namespace b200sr
-
-extern "C" int b200sr_conv3x3_small(const void* x, const void* w, const float* bias, const void* addend, void* y,
-                                    int32_t N, int32_t H, int32_t W, int32_t Cin, int32_t Cout, int32_t out_nchw_f32,
-                                    void* stream_ptr) {
-  if (x == nullptr || w == nullptr || y == nullptr) return B200SR_EINVAL;
-  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
-  if (N <= 0 || H <= 0 || W <= 0 || Cin <= 0 || Cout <= 0) return B200SR_EINVAL;
-  const __nv_bfloat16* xi = reinterpret_cast<const __nv_bfloat16*>(x);
-  const __nv_bfloat16* wi = reinterpret_cast<const __nv_bfloat16*>(w);
-  if (Cin <= 8 && (Cout % 8) == 0) {
-    if (out_nchw_f32) return B200SR_EINVAL;
-    const size_t smem = static_cast<size_t>(Cout) * 9 * Cin * sizeof(float);
-    if (smem > 96 * 1024) return B200SR_EINVAL;
-    static bool attr_set[64] = {false};  // the attribute is per device
-    if (first_use_on_device(attr_set))
-      cudaFuncSetAttribute(conv3x3_few_in_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-    const size_t total = static_cast<size_t>(N) * H * W * (Cout / 8);
-    int grid = static_cast<int>((total + 255) / 256);
-    if (grid > num_sms() * 4) grid = num_sms() * 4;
-    launch_k(conv3x3_few_in_kernel, dim3(grid), dim3(256), smem, stream, 1, xi, wi, bias, reinterpret_cast<const __nv_bfloat16*>(addend),
-                                                       reinterpret_cast<__nv_bfloat16*>(y), N, H, W, Cin, Cout);
-  } else if (Cout <= 4 && (Cin % 8) == 0) {
-    if (addend != nullptr) return B200SR_EINVAL;
-    const size_t total = static_cast<size_t>(N) * H * W;
-    int grid = static_cast<int>((total + 7) / 8);
-    if (grid > num_sms() * 32) grid = num_sms() * 32;
-    switch (Cout) {
-      case 1: launch_k(conv3x3_few_out_kernel<1>, dim3(grid), dim3(256), 0, stream, 1, xi, wi, bias, y, N, H, W, Cin, out_nchw_f32); break;
-      case 2: launch_k(conv3x3_few_out_kernel<2>, dim3(grid), dim3(256), 0, stream, 1, xi, wi, bias, y, N, H, W, Cin, out_nchw_f32); break;
-      case 3: launch_k(conv3x3_few_out_kernel<3>, dim3(grid), dim3(256), 0, stream, 1, xi, wi, bias, y, N, H, W, Cin, out_nchw_f32); break;
-      default: launch_k(conv3x3_few_out_kernel<4>, dim3(grid), dim3(256), 0, stream, 1, xi, wi, bias, y, N, H, W, Cin, out_nchw_f32); break;
-    }
-  } else {
-    return B200SR_EINVAL;
-  }
   return cudaGetLastError() == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
 }
 

@@ -725,85 +725,6 @@ extern "C" int b200sr_layer_norm(const void* x, void* y, const float* weight, co
 
 namespace b200sr {
 
-// ------------------------------------------------------------------------------------------
-// Row softmax of an fp32 [rows, cols] score matrix -> bf16 probabilities (SR3 single-head
-// attention, models/sr3_model/sr3_modules/unet.py:133-138).  One warp per row, three passes
-// over an L2-resident row.
-// ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-softmax_rows_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ y, int rows, int cols, int valid,
-                    float scale) {
-  pdl_launch_dependents();
-  pdl_wait();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int row = blockIdx.x * (blockDim.x >> 5) + warp;
-  if (row >= rows) return;
-  const float* src = x + static_cast<size_t>(row) * cols;
-  float mx = -INFINITY;
-  for (int c = lane; c < valid; c += 32) mx = fmaxf(mx, src[c]);
-  mx = warp_max(mx) * scale;
-  float sum = 0.f;
-  for (int c = lane; c < valid; c += 32) sum += __expf(src[c] * scale - mx);
-  const float inv = 1.0f / warp_sum(sum);
-  __nv_bfloat16* dst = y + static_cast<size_t>(row) * cols;
-  for (int c = lane; c < cols; c += 32)
-    dst[c] = __float2bfloat16(c < valid ? __expf(src[c] * scale - mx) * inv : 0.f);  // padded keys get weight 0
-}
-
-// Long rows (1024 < cols <= 32768, cols % 4 == 0): one CTA per row, the row is read ONCE into registers (64 floats per
-// thread), maximum and sum are block reductions, the probabilities are written once: 4 + 2 bytes per element instead
-// of three passes over a row that no longer fits L1 (T = 16384 keys: 64 KB per row, 1 GB per score matrix).
-template <int THREADS>
-__global__ void __launch_bounds__(THREADS)
-softmax_rows_block_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ y, int cols, int valid, float scale) {
-  pdl_launch_dependents();
-  pdl_wait();
-  __shared__ float s_red[32];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
-  const size_t row = blockIdx.x;
-  const float4* src = reinterpret_cast<const float4*>(x + row * cols);
-  const int c4 = cols >> 2;
-  float4 v[16];
-  float mx = -INFINITY;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    const int idx = threadIdx.x + i * blockDim.x;
-    v[i] = idx < c4 ? __ldcs(src + idx) : make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
-    const int c = idx * 4;
-    if (c + 0 >= valid) v[i].x = -INFINITY;
-    if (c + 1 >= valid) v[i].y = -INFINITY;
-    if (c + 2 >= valid) v[i].z = -INFINITY;
-    if (c + 3 >= valid) v[i].w = -INFINITY;
-    mx = fmaxf(mx, fmaxf(fmaxf(v[i].x, v[i].y), fmaxf(v[i].z, v[i].w)));
-  }
-  mx = warp_max(mx);
-  if (lane == 0) s_red[warp] = mx;
-  __syncthreads();
-  mx = lane < nwarps ? s_red[lane] : -INFINITY;
-  mx = warp_max(mx) * scale;
-  __syncthreads();
-  float sum = 0.f;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    v[i].x = __expf(v[i].x * scale - mx);
-    v[i].y = __expf(v[i].y * scale - mx);
-    v[i].z = __expf(v[i].z * scale - mx);
-    v[i].w = __expf(v[i].w * scale - mx);
-    sum += (v[i].x + v[i].y) + (v[i].z + v[i].w);
-  }
-  sum = warp_sum(sum);
-  if (lane == 0) s_red[warp] = sum;
-  __syncthreads();
-  sum = lane < nwarps ? s_red[lane] : 0.f;
-  const float inv = 1.0f / warp_sum(sum);
-  uint2* dst = reinterpret_cast<uint2*>(y + row * cols);
-#pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    const int idx = threadIdx.x + i * blockDim.x;
-    if (idx < c4) dst[idx] = make_uint2(pack_bf16x2(v[i].x * inv, v[i].y * inv), pack_bf16x2(v[i].z * inv, v[i].w * inv));
-  }
-}
-
 // Two-pass row softmax (b200sr_gemm_bf16 with row_softmax = 1 / 2): fold the per-N-tile (max, sum of 2^(x - max)) pairs of
 // pass 1 into one (M, L) pair per row, so that pass 2 reads 8 bytes per row instead of chaining `parts` dependent updates
 // in front of every tile's epilogue (measured: 705 us instead of ~200 for the 16384 x 16384 apply pass).
@@ -833,28 +754,6 @@ extern "C" int b200sr_row_softmax_fold(const float* parts, int32_t n_parts, int6
   const unsigned grid = static_cast<unsigned>((rows + 255) / 256);
   return launch_k(row_softmax_fold_kernel, dim3(grid), dim3(256), 0, stream, 1, reinterpret_cast<const float2*>(parts), n_parts,
                   rows, reinterpret_cast<float2*>(out)) == cudaSuccess
-             ? B200SR_OK
-             : B200SR_ELAUNCH;
-}
-
-extern "C" int b200sr_softmax_rows(const float* x, void* y, int32_t rows, int32_t cols, int32_t valid, float scale,
-                                   void* stream_ptr) {
-  if (x == nullptr || y == nullptr) return B200SR_EINVAL;
-  const cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
-  if (rows <= 0 || cols <= 0 || valid <= 0 || valid > cols) return B200SR_EINVAL;
-  if (cols > 1024 && cols <= 32768 && (cols % 4) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
-      (reinterpret_cast<uintptr_t>(y) & 7) == 0) {
-    int threads = ((cols / 4 + 15) / 16 + 31) / 32 * 32;   // 16 float4 per thread
-    if (threads < 64) threads = 64;
-    __nv_bfloat16* yo = reinterpret_cast<__nv_bfloat16*>(y);
-    const cudaError_t err =
-        threads <= 256 ? launch_k(softmax_rows_block_kernel<256>, dim3(rows), dim3(threads), 0, stream, 1, x, yo, cols, valid, scale)
-                       : launch_k(softmax_rows_block_kernel<512>, dim3(rows), dim3(threads), 0, stream, 1, x, yo, cols, valid, scale);
-    return err == cudaSuccess ? B200SR_OK : B200SR_ELAUNCH;
-  }
-  const int grid = (rows + 7) / 8;
-  return launch_k(softmax_rows_kernel, dim3(grid), dim3(256), 0, stream, 1, x, reinterpret_cast<__nv_bfloat16*>(y), rows,
-                  cols, valid, scale) == cudaSuccess
              ? B200SR_OK
              : B200SR_ELAUNCH;
 }

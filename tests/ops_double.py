@@ -79,7 +79,7 @@ def gemm(a, w, bias=None, *, residual=None, rowvec=None, rows_per_group=0, geglu
 
 def gemm_row_softmax(a, w, scale, valid_cols=None, w_dynamic=True):
     s = a.float().reshape(-1, a.shape[-1]) @ w.float().t()
-    return softmax_rows(s, scale, valid_cols=valid_cols)
+    return _softmax_rows(s, scale, valid_cols=valid_cols)
 
 
 class RowStats:
@@ -135,18 +135,6 @@ def conv3x3(x, w, bias=None, *, stride=1, rowvec=None, residual=None, alpha=1.0,
     return y
 
 
-def conv3x3_small(x, w, bias, *, addend=None, out_nchw_f32=False):
-    cout, cin = w.shape[0], x.shape[-1]
-    w4 = w.float().view(cout, 3, 3, cin).permute(0, 3, 1, 2)
-    y = F.conv2d(x.float().permute(0, 3, 1, 2), w4, bias, padding=1)
-    if out_nchw_f32:
-        return y.contiguous()
-    y = y.permute(0, 2, 3, 1)
-    if addend is not None:
-        y = y + addend.float()
-    return y.to(bf16).contiguous()
-
-
 def group_norm(x, weight, bias, *, groups=32, eps=1e-5, silu=False, sft_gamma=None, sft_beta=None, raw=None,
                control_scale=1.0):
     shape = x.shape
@@ -182,14 +170,14 @@ def attention(q, k, v, heads, *, q_col=0, k_col=0, v_col=0, scale=None, causal=F
 
 def single_head_attention(q, k, v_t, scale, out_bias=None, valid_keys=None):
     s = q.float() @ k.float().t()
-    p = softmax_rows(s, scale, valid_cols=valid_keys).float()
+    p = _softmax_rows(s, scale, valid_cols=valid_keys).float()
     o = p @ v_t.float().t()
     if out_bias is not None:
         o = o + out_bias
     return o.to(bf16)
 
 
-def softmax_rows(x, scale=1.0, valid_cols=None):
+def _softmax_rows(x, scale=1.0, valid_cols=None):
     v = x.shape[-1] if valid_cols is None else valid_cols
     y = torch.zeros_like(x, dtype=torch.float32)
     y[..., :v] = torch.softmax(x.float()[..., :v] * scale, dim=-1)
@@ -198,10 +186,6 @@ def softmax_rows(x, scale=1.0, valid_cols=None):
 
 def nchw_to_nhwc_bf16(x, scale=1.0):
     return (x * scale).to(bf16).permute(0, 2, 3, 1).contiguous()
-
-
-def nhwc_to_nchw_f32(x):
-    return x.float().permute(0, 3, 1, 2).contiguous()
 
 
 def cast_bf16(x):

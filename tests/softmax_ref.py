@@ -140,28 +140,8 @@ def attention_logits(q, k, heads: int, b: int, h: int, scale: float = 0.125, col
 
 
 # ------------------------------------------------------------------------------------------------------------------------
-# whole-row softmax: ops.softmax_rows, ops.gemm_row_softmax, ops.single_head_attention
+# whole-row softmax: ops.gemm_row_softmax, ops.single_head_attention
 # ------------------------------------------------------------------------------------------------------------------------
-def softmax_rows(x: torch.Tensor, scale: float = 1.0, valid_cols=None):
-    """softmax(x * scale) over the first ``valid_cols`` columns of fp32 rows (others exactly 0): (ref, bound).
-
-    The kernels take ``__expf(x * scale - max)`` and an fp32 sum: per lane ``valid / 32`` terms then a warp tree (warp
-    kernel), or 64 per thread then warp and block trees (block kernel) -- a chain of at most ``max(valid / 32, 64) + 16``
-    roundings.  Logit error: 2^-21 max|t| (``x * scale``, the subtraction, the ``* log2 e`` inside ``__expf``)."""
-    x2 = x.reshape(-1, x.shape[-1]).to(f64)
-    cols = x2.shape[1]
-    valid = cols if valid_cols is None else int(valid_cols)
-    t = x2[:, :valid] * (scale * LOG2E)
-    p = _softmax2(t)
-    delta = 2.0 ** -21 * t.abs().amax(1, keepdim=True)
-    n_sum = max(math.ceil(valid / 32), 64) + 16
-    ref = torch.zeros_like(x2)
-    bound = torch.zeros_like(x2)
-    ref[:, :valid] = p
-    bound[:, :valid] = _prob_bound(p, delta, n_sum * U_F32 / EX2)
-    return ref.reshape(x.shape), bound.reshape(x.shape)
-
-
 def gemm_row_softmax(a: torch.Tensor, w: torch.Tensor, scale: float, valid_cols=None):
     """softmax(scale * a @ w^T) over the first ``valid_cols`` columns of each row (others exactly 0): (ref, bound).
 
@@ -528,13 +508,3 @@ def row_softmax_inputs(M: int, N: int, K: int, tile: int, far: float = 140.0, se
     w[torch.arange(N), 2 * nt + 1] = 1.0
     w[:, 2 * n_tiles:] = torch.randn(N, nd, generator=g, dtype=f64)
     return a.to(bf16), w.to(bf16)
-
-
-def wide_range_rows(rows: int, cols: int, log2_range: float, seed: int = 0) -> torch.Tensor:
-    """fp32 [rows, cols] logits (natural units, for softmax_rows at scale 1) spanning ``log2_range`` log2 units per row:
-    a uniform spread, with the maximum placed at a row-dependent column (first, last, or inside)."""
-    g = torch.Generator().manual_seed(seed)
-    x = torch.rand(rows, cols, generator=g, dtype=f64) * (log2_range / LOG2E) - log2_range / LOG2E
-    hot = torch.tensor([0, cols - 1, cols // 2, cols // 3])[torch.arange(rows) % 4]
-    x[torch.arange(rows), hot] = 0.5
-    return x.to(torch.float32)

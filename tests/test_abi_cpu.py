@@ -104,16 +104,13 @@ def test_abi_version_matches_the_header():
 NULL_REJECTED = {
     "b200sr_gemm_bf16": ("A W epi", dict(lda=64, M=128, N=64, K=64, force_bn=0)),
     "b200sr_conv3x3_bf16": ("x w epi", dict(N=1, H=16, W=16, Cin=64, Cout=64, stride=1, pad_lo=1, force_bn=0)),
-    "b200sr_conv3x3_small": ("x w y", dict(N=1, H=8, W=8, Cin=4, Cout=64, out_nchw_f32=0)),
     "b200sr_group_norm_nhwc": ("x y", dict(N=1, HW=64, C=64, groups=32, eps=1e-5, silu=0, control_scale=1.0)),
     "b200sr_group_norm_stats": ("x", dict(N=1, HW=64, C=64, groups=32, eps=1e-5)),
     "b200sr_layer_norm": ("x y", dict(M=8, C=64, eps=1e-5)),
     "b200sr_attention_d64": ("q k v out", dict(ldq=64, q_col=0, ldk=64, k_col=0, ldv=64, v_col=0, ldo=64, B=1, H=1,
                                                Nq=128, Nk=128, scale=0.125, causal=0)),
     "b200sr_row_softmax_fold": ("parts out", dict(n_parts=2, rows=128)),
-    "b200sr_softmax_rows": ("x y", dict(rows=8, cols=128, valid_cols=77, scale=0.125)),
     "b200sr_nchw_f32_to_nhwc_bf16": ("x y", dict(N=1, C=4, HW=64, scale=1.0)),
-    "b200sr_nhwc_bf16_to_nchw_f32": ("x y", dict(N=1, C=4, HW=64)),
     "b200sr_nhwc_bf16_to_nchw_f32_strided": ("x y", dict(N=1, C=4, Cs=8, HW=64)),
     "b200sr_upsample2x_nhwc": ("x y", dict(N=1, H=8, W=8, C=64)),
     "b200sr_concat_add": ("a b out", dict(Ca=64, Cb=64, rows=64)),
@@ -157,7 +154,7 @@ print(json.dumps([getattr(lib, name)(*[structs.get(a, a) if isinstance(a, str) e
 """
 
 
-def test_null_pointers_are_rejected_before_any_cuda_call(lib):
+def test_entry_points_reject_null_pointers_before_any_cuda_call(lib):
     """Each pointer an entry point rejects as NULL gives -22 (EINVAL) with every other argument valid, checked before
     the entry point touches the CUDA runtime: the calls run without a device."""
     protos = prototypes()

@@ -1,5 +1,5 @@
-"""GPU parity of the round-2 operator additions against plain torch fp32 references: row softmax (warp-per-row and the
-single-pass CTA-per-row kernel for long rows), the chunked single-head attention helper, copy_batch, weighted strips."""
+"""GPU parity of the round-2 operator additions against plain torch fp32 references: the chunked single-head attention
+helper, copy_batch, weighted strips."""
 import pytest
 import torch
 
@@ -10,21 +10,6 @@ bf16 = torch.bfloat16
 def rel_l2(a, b):
     a, b = a.float(), b.float()
     return ((a - b).norm() / (b.norm() + 1e-12)).item()
-
-
-@pytest.mark.parametrize("rows,cols,valid", [(37, 80, 77), (64, 1024, 1024), (33, 4096, 4096), (16, 16384, 16384),
-                                             (8, 16384, 16001), (4, 32768, 32768), (3, 65536, 65536), (5, 1028, 1000)])
-def test_softmax_rows(rows, cols, valid):
-    from b200sr import ops
-
-    g = torch.Generator(device="cuda").manual_seed(rows * 7 + cols)
-    x = torch.randn(rows, cols, generator=g, device="cuda") * 6
-    y = ops.softmax_rows(x, 0.37, valid_cols=valid)
-    ref = torch.zeros_like(x)
-    ref[:, :valid] = torch.softmax(x[:, :valid] * 0.37, dim=-1)
-    assert y.dtype == bf16 and torch.equal(y[:, valid:], torch.zeros_like(y[:, valid:]))
-    assert rel_l2(y, ref) < 4e-3
-    assert torch.allclose(y.float().sum(-1), torch.ones(rows, device="cuda"), atol=2e-2)
 
 
 @pytest.mark.parametrize("t,chunk", [(1024, 1 << 30), (4096, 4 * 4096 * 1024)])
@@ -241,7 +226,7 @@ def test_two_pass_row_softmax_gemm(m, n, valid):
     assert worst < 4e-3, worst
 
 
-def test_single_head_attention_two_pass_equals_three_kernel_form(monkeypatch):
+def test_single_head_attention_with_bias():
     from b200sr import ops
 
     g = torch.Generator(device="cuda").manual_seed(11)
@@ -249,9 +234,6 @@ def test_single_head_attention_two_pass_equals_three_kernel_form(monkeypatch):
     q, k, v = ((torch.randn(t, c, generator=g, device="cuda") * 0.5).to(bf16) for _ in range(3))
     bias = torch.randn(c, generator=g, device="cuda")
     v_t = v.t().contiguous()
-    monkeypatch.setattr(ops, "TWO_PASS_SOFTMAX", True)
     a = ops.single_head_attention(q, k, v_t, c ** -0.5, bias)
-    monkeypatch.setattr(ops, "TWO_PASS_SOFTMAX", False)
-    b = ops.single_head_attention(q, k, v_t, c ** -0.5, bias)
     ref = torch.softmax(q.float() @ k.float().t() * c ** -0.5, dim=-1) @ v.float() + bias
-    assert rel_l2(a, ref) < 6e-3 and rel_l2(b, ref) < 6e-3 and rel_l2(a, b) < 4e-3
+    assert rel_l2(a, ref) < 6e-3

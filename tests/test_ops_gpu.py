@@ -113,26 +113,6 @@ def test_conv3x3(ops, N, H, W, Cin, Cout, stride):
     assert rel_l2(out.permute(0, 3, 1, 2), ref) < 5e-3
 
 
-def test_conv3x3_small(ops):
-    x = _rand(2, 4, 32, 32, seed=1).to(bf16)
-    w = _rand(320, 4, 3, 3, seed=2) / 6.0
-    b = _rand(320, seed=3)
-    add = _rand(2, 32, 32, 320, seed=4).to(bf16)
-    out = ops.conv3x3_small(x.permute(0, 2, 3, 1).contiguous(), ops.pack_conv3x3(w), b, addend=add)
-    ref = F.conv2d(x.float(), w.to(bf16).float(), b, padding=1) + add.float().permute(0, 3, 1, 2)
-    assert rel_l2(out.permute(0, 3, 1, 2), ref) < 5e-3
-    x = _rand(2, 320, 32, 32, seed=5).to(bf16)
-    w = _rand(4, 320, 3, 3, seed=6) / math.sqrt(2880)
-    b = _rand(4, seed=7)
-    out = ops.conv3x3_small(x.permute(0, 2, 3, 1).contiguous(), ops.pack_conv3x3(w), b, out_nchw_f32=True)
-    ref = F.conv2d(x.float(), w.to(bf16).float(), b, padding=1)
-    assert out.dtype == torch.float32 and rel_l2(out, ref) < 2e-3
-    w3 = _rand(3, 64, 3, 3, seed=8) / 24.0
-    x3 = _rand(1, 64, 16, 16, seed=9).to(bf16)
-    out = ops.conv3x3_small(x3.permute(0, 2, 3, 1).contiguous(), ops.pack_conv3x3(w3), None)
-    assert rel_l2(out.permute(0, 3, 1, 2), F.conv2d(x3.float(), w3.to(bf16).float(), None, padding=1)) < 5e-3
-
-
 @pytest.mark.parametrize("N,H,W,C,eps,silu", [(2, 128, 128, 320, 1e-5, True), (2, 32, 32, 1280, 1e-6, False),
                                               (2, 32, 32, 2560, 1e-5, True), (1, 16, 16, 64, 1e-5, True),
                                               (3, 8, 8, 960, 1e-5, True), (2, 64, 64, 1920, 1e-5, False)])
@@ -263,12 +243,17 @@ def test_attention_split_is_deterministic_and_leaves_counters_zero(ops):
         assert int(w[:512].view(torch.int32).abs().sum()) == 0
 
 
-def test_layout_upsample_concat_misc(ops):
+def test_layout_strided_upsample_concat_misc(ops):
     x = _rand(2, 4, 16, 24, seed=1)
     y = ops.nchw_to_nhwc_bf16(x, 0.5)
     assert torch.equal(y, (x * 0.5).to(bf16).permute(0, 2, 3, 1).contiguous())
     z = _rand(2, 16, 24, 320, seed=2).to(bf16)
-    assert torch.equal(ops.nhwc_to_nchw_f32(z), z.float().permute(0, 3, 1, 2).contiguous())
+    from b200sr import _lib
+    for c in (4, 320):   # the first 4 of 320 channels: the stride of the <= 4-channel convolutions' padded output
+        y = torch.empty(2, c, 16, 24, device="cuda")
+        assert _lib.load().b200sr_nhwc_bf16_to_nchw_f32_strided(z.data_ptr(), y.data_ptr(), 2, c, 320, 16 * 24,
+                                                                ops._stream()) == 0
+        assert torch.equal(y, z[..., :c].float().permute(0, 3, 1, 2).contiguous())
     up = ops.upsample2x(z)
     ref = F.interpolate(z.float().permute(0, 3, 1, 2), scale_factor=2, mode="nearest").permute(0, 2, 3, 1).to(bf16)
     assert torch.equal(up, ref.contiguous())

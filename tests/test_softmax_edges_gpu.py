@@ -1,8 +1,8 @@
 """Every softmax path of the library against float64, element by element, on inputs designed to reach its rescale and
 merge code: the attention kernel's lazy rescale and split merge, the per-head segment softmax epilogue (with and without
-the LayerNorm fold), the two-pass whole-row softmax of the GEMM, both row-softmax kernels, and CUDA-graph replays of the
-stateful ones.  References, bounds (derived in softmax_ref's docstrings) and generators live in tests/softmax_ref.py;
-each test prints its worst err / bound."""
+the LayerNorm fold), the two-pass whole-row softmax of the GEMM, and CUDA-graph replays of the stateful ones.
+References, bounds (derived in softmax_ref's docstrings) and generators live in tests/softmax_ref.py; each test prints its
+worst err / bound."""
 import pytest
 import torch
 
@@ -143,7 +143,7 @@ def test_head_softmax_epilogue(ops, heads, valid, log2_range, ln):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# whole-row softmax: two-pass GEMM, both row-softmax kernels, chunked single-head attention
+# whole-row softmax: two-pass GEMM, chunked single-head attention
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("M,N,cut", [(1000, 2048, "tile"), (1000, 2048, "inside"), (1000, 2048, "one"), (700, 4104, None)])
 def test_gemm_row_softmax_far_apart_tiles(ops, M, N, cut):
@@ -159,34 +159,6 @@ def test_gemm_row_softmax_far_apart_tiles(ops, M, N, cut):
         assert bool((p[:, 0] == 1.0).all())
     what = f"gemm_row_softmax M={M} N={N} tile={tile} valid={valid}"
     _report(what, sr.assert_within(p, ref, bound, what))
-
-
-def _softmax_rows_kernel(x: torch.Tensor) -> str:
-    """Which kernel norm.cu's softmax_rows picks for this input (the output is freshly allocated, hence aligned)."""
-    cols = x.shape[-1]
-    return "block" if 1024 < cols <= 32768 and cols % 4 == 0 and x.data_ptr() % 16 == 0 else "warp"
-
-
-@pytest.mark.parametrize("rows,cols,valid,offset,kernel", [
-    (64, 1024, 1, 0, "warp"),
-    (40, 1028, 1000, 0, "block"),
-    (8, 32768, 32768, 0, "block"),
-    (8, 32772, 30001, 0, "warp"),      # longer than the block kernel holds
-    (16, 4099, 4099, 0, "warp"),       # cols % 4 != 0
-    (16, 4096, 4000, 1, "warp"),       # a view one float into its buffer: not 16-byte aligned
-    (16, 4096, 4000, 0, "block"),
-])
-def test_softmax_rows_wide_range(ops, rows, cols, valid, offset, kernel):
-    data = sr.wide_range_rows(rows, cols, 200.0, seed=cols + offset).cuda()
-    buf = torch.empty(rows * cols + 4, device="cuda")
-    x = buf[offset:offset + rows * cols].view(rows, cols)
-    x.copy_(data)
-    assert _softmax_rows_kernel(x) == kernel
-    y = ops.softmax_rows(x, 1.0, valid_cols=valid)
-    ref, bound = sr.softmax_rows(data, 1.0, valid)
-    assert bool((y[:, valid:] == 0).all())
-    what = f"softmax_rows {rows}x{cols} valid={valid} ({kernel} kernel)"
-    _report(what, sr.assert_within(y, ref, bound, what))
 
 
 def test_single_head_attention_valid_keys_across_query_chunks(ops, monkeypatch):

@@ -123,18 +123,13 @@ if which == "scores":
 if which == "rowsoftmax":
     for (M, N, K) in ((16384, 16384, 512), (4096, 4096, 512)):
         q = r(M, K); k_ = r(N, K); v_t = r(K, N)
-        sc = torch.empty(M, N, device=dev); o = torch.empty(M, K, device=dev, dtype=bf16)
-        def three(i):
-            ops.gemm(q, k_, out=sc, out_fp32=True, w_dynamic=True)
-            p_ = ops.softmax_rows(sc, K ** -0.5)
-            ops.gemm(p_, v_t, None, w_dynamic=True, out=o)
+        o = torch.empty(M, K, device=dev, dtype=bf16)
         def two(i):
             p_ = ops.gemm_row_softmax(q, k_, K ** -0.5)
             ops.gemm(p_, v_t, None, w_dynamic=True, out=o)
-        t3 = graph_time(three); t2 = graph_time(two)
+        t2 = graph_time(two)
         t1 = graph_time(lambda i: ops.gemm_row_softmax(q, k_, K ** -0.5))
-        print(f"single-head attention T{M} C{K}: score GEMM + softmax + PV {t3:8.1f} us | two-pass softmax GEMM + PV {t2:8.1f} us "
-              f"(the two passes alone {t1:8.1f} us)")
+        print(f"single-head attention T{M} C{K}: two-pass softmax GEMM + PV {t2:8.1f} us (the two passes alone {t1:8.1f} us)")
 if which == "lnfold":
     # (1) single GEMMs back to back: plain / writing row statistics / LayerNorm folded in / both
     for (M, N, K, geglu, residual) in ((2048, 1280, 1280, False, True), (2048, 3840, 1280, False, False),
@@ -174,7 +169,7 @@ if which == "lnfold":
                 x, st = rr if fused else (rr, None)
             return x
         res_ = {}
-        for fused in ((True, False) if md.FUSE_LN_INTO_GEMM else (False,)):
+        for fused in (True, False):
             with torch.no_grad():
                 y = run(fused); torch.cuda.synchronize()
                 g = torch.cuda.CUDAGraph()
@@ -188,8 +183,7 @@ if which == "lnfold":
                 e1.record(); torch.cuda.synchronize()
                 res_[fused] = (e0.elapsed_time(e1) / 10 / nblk * 1e3, y.float().clone())
         msg = " | ".join(f"{'folded' if k else 'LayerNorm kernels'} {v[0]:7.1f} us/block" for k, v in res_.items())
-        if len(res_) == 2:
-            msg += f" | rel diff {((res_[True][1] - res_[False][1]).norm() / res_[False][1].norm()).item():.2e}"
+        msg += f" | rel diff {((res_[True][1] - res_[False][1]).norm() / res_[False][1].norm()).item():.2e}"
         print(f"transformer block B{B} T{T} C{C}: {msg}")
 tot = 0.0
 print(f"{'op':46s} {'us/launch':>9s} {'TF/s|TB/s':>9s} {'n/step':>6s} {'ms/step':>8s}")
